@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- MALI ray-depth updates/s on B200 (BASELINE.json metric), one process per GPU.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--ncol C] [--iters I]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--ncol C] [--iters I] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P \
         bench.py --gpus N --steps K --warmup W
     python bench.py --workload lambda_shard [--gpus N]        # BASELINE config 5 experiment (one column, wavelength-sharded)
@@ -213,7 +213,8 @@ def run_lambda_shard(args):
     """BASELINE config 5 (an experiment, not the production path): one stress column -- 10x refined wavelength grid,
     10-point quadrature, 512 depths -- split over the GPUs by wavelength (ranges balanced by work); every iteration exchanges Gamma (one NCCL all-gather of
     [Gamma | dJ] + a fixed-order sum, lambda_shard.GammaExchange).
-    A step is one MALI iteration of the column (strong scaling: the column is fixed)."""
+    A step is one MALI iteration of the column (strong scaling: the column is fixed); a warm-up pass of --warmup
+    iterations precedes the --steps timed ones."""
     sys.path.insert(0, os.path.join(ROOT, 'tools'))
     import lambda_shard_experiment as ls
     world = int(os.environ.get('WORLD_SIZE', '1'))
@@ -226,10 +227,10 @@ def run_lambda_shard(args):
         json_fd = os.dup(1)
         os.dup2(2, 1)
     q = ls.build_problem()
-    out = ls.run(q, iters=max(6, args.steps))
+    out = ls.run(q, iters=args.steps, warmup=args.warmup)
     if rank == 0:
-        line = {'metric': METRIC, 'value': out['updates_per_s'], 'unit': UNIT, 'n_gpus': world, 'steps': max(6, args.steps),
-                'warmup': max(6, args.steps), 'ms_per_step': out['ms_per_iteration'], 'higher_is_better': True,
+        line = {'metric': METRIC, 'value': out['updates_per_s'], 'unit': UNIT, 'n_gpus': world, 'steps': args.steps,
+                'warmup': args.warmup, 'ms_per_step': out['ms_per_iteration'], 'higher_is_better': True,
                 'scaling': 'strong', 'vs_baseline': None, 'dtype': 'f64', 'data': 'synthetic',
                 'config': {'workload': 'EXPERIMENT: wavelength-sharded single stress column (BASELINE config 5), Gamma '
                                        'exchange (one NCCL all-gather + fixed-order sum) every iteration', 'Nspect': out['Nspect'], 'Nrays': out['Nrays'],
@@ -242,6 +243,41 @@ def run_lambda_shard(args):
     import torch.distributed as dist
     if dist.is_initialized():
         dist.destroy_process_group()
+
+
+DUMP_BYTES = 60 * 10**6      # array bytes of --dump-outputs: with the .npy headers, under 64 MB
+
+
+def dump_outputs(out_dir, eng, col_global0, world, rank):
+    """Writes what the resident solve hands its caller, in the reference's shapes and float64: emergent intensity
+    I [col, Nspect, Nrays], populations n [col, sum Nlevel, Nspace], dJ and dPops [col] with `columns`, the global
+    index of each column, and the mean intensity J [col, Nspect, Nspace] with `J_columns`.  At most DUMP_BYTES in all
+    (two thirds of it at most for I, n, dJ, dPops, the rest for J, which is 13x larger per column): what does not fit
+    is represented by a fixed, seeded sample of the columns.  With several ranks each writes its share of the budget
+    as <name>_rank<r>.npy."""
+    import torch
+    mt, ncol = eng.mt, eng.ncol
+    rng = np.random.default_rng(0)
+
+    def sample(bytes_per_col, budget):
+        k = min(ncol, budget // bytes_per_col)
+        return np.arange(ncol) if k == ncol else np.sort(rng.choice(ncol, k, replace=False))
+
+    budget = DUMP_BYTES // world
+    per_col = 8 * (mt.Nspect * mt.Nrays + eng.lay.pops + 3)
+    cols = sample(per_col, 2 * budget // 3)
+    jcols = sample(8 * (mt.Nspect * mt.Nspace + 1), budget - len(cols) * per_col)
+    idx, jidx = (torch.from_numpy(c).to(eng.device) for c in (cols, jcols))
+    out = {'columns': torch.from_numpy((col_global0 + cols).astype(np.float64)),
+           'I': eng.t_I.view(ncol, mt.Nspect, mt.Nrays).index_select(0, idx),
+           'n': eng.t_pops.view(ncol, -1, mt.Nspace).index_select(0, idx),
+           'dJ': eng.t_dJ.index_select(0, idx), 'dPops': eng.t_dPops.index_select(0, idx),
+           'J_columns': torch.from_numpy((col_global0 + jcols).astype(np.float64)),
+           'J': eng.t_J.view(ncol, mt.Nspace, mt.Nspect).index_select(0, jidx).transpose(1, 2)}
+    os.makedirs(out_dir, exist_ok=True)
+    suffix = '_rank%d' % rank if world > 1 else ''
+    for name, t in out.items():
+        np.save(os.path.join(out_dir, name + suffix + '.npy'), np.ascontiguousarray(t.cpu().numpy()))
 
 
 def workload_config(args, base):
@@ -269,7 +305,7 @@ def main():
     ap.add_argument('--iters', type=int, default=16, help='MALI iterations per solve (= per step)')
     ap.add_argument('--fixture', default='c2_falc_cah')
     ap.add_argument('--chunk', type=int, default=512, help='columns per upload chunk in the e2e path')
-    ap.add_argument('--e2e-steps', type=int, default=0, help='timed steps of the e2e paths (default: min(steps, 3))')
+    ap.add_argument('--e2e-steps', type=int, default=0, help='timed steps of the e2e paths (default: --steps)')
     ap.add_argument('--first-chunk', type=int, default=0,
                     help='e2e path: size of a smaller first chunk (shortens the exposed first host->device copy)')
     ap.add_argument('--sched', default='',
@@ -282,7 +318,13 @@ def main():
                          'stress column wavelength-sharded over the GPUs with a Gamma all-reduce per iteration')
     ap.add_argument('--no-e2e', action='store_true')
     ap.add_argument('--no-cpu', action='store_true')
+    ap.add_argument('--dump-outputs', metavar='DIR', default=None,
+                    help='write what the timed resident solve computed in its last step to DIR/<name>.npy')
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
+    if args.dump_outputs and (args.impl != 'ours' or args.workload != 'columns'):
+        ap.error('--dump-outputs applies to the column workload of --impl ours')
     args.warmup = max(args.warmup, 0)
     base = load_base(args.fixture)
 
@@ -403,6 +445,8 @@ def main():
     launches = eng.launch_count() - launches0
     clocks = sampler.stop() if sampler else None
     finite = bool(torch.isfinite(eng.t_pops).all().item() and torch.isfinite(eng.t_I).all().item())
+    if args.dump_outputs:      # before the side sections below run the solve again
+        dump_outputs(args.dump_outputs, eng, col_global0, world, rank)
     total_units = world * ncol * units_per_col_iter * iters * args.steps
     value = total_units / (ms * 1e-3)
 
@@ -544,7 +588,7 @@ def main():
         solve_from_host()
         barrier()
         l0 = eng.launch_count()
-        k_e2e = args.e2e_steps if args.e2e_steps > 0 else max(1, min(args.steps, 3))
+        k_e2e = args.e2e_steps if args.e2e_steps > 0 else args.steps
         e0.record()
         for _ in range(k_e2e):
             solve_from_host()

@@ -4,15 +4,18 @@ The fast formal-solution kernels are specialised on the *structure* of a wavelen
 it and which atomic levels they share; csrc/mali_fs_spec.cuh).  libmali_b200.so ships instances for the models of the
 committed fixtures; any other model still runs -- on the generic kernel, a few times slower.  This module closes the
 gap when nvcc is available: it lists the tile structures of a model, writes an instance file for them and builds a
-model-specific variant of the library (same C ABI) next to the stock one, cached by content hash.
+model-specific variant of the library (same C ABI), cached under a hash of its structures, sources and compiler
+options in a private per-user temporary directory (the package tree is left as the build left it; it may be read-only).
 
     lib_path = specialize.library_for(problem)      # None when nothing had to be (or could be) built
     eng = MaliEngine(problem, ncol, specialize=True)   # does it for you
 """
+import fcntl
 import hashlib
 import os
-import shutil
+import stat
 import sys
+import tempfile
 
 import numpy as np
 
@@ -70,6 +73,32 @@ def stock_keys():
     return keys
 
 
+def cache_dir():
+    """Per-user directory of the model-specific libraries built at run time.  Libraries found there are loaded, so
+    it must be this user's own private directory (a predictable name in a shared temporary directory)."""
+    d = os.path.join(tempfile.gettempdir(), 'lightspinner_b200-%d' % os.getuid())
+    try:
+        os.mkdir(d, 0o700)
+    except FileExistsError:
+        pass
+    st = os.lstat(d)
+    if not stat.S_ISDIR(st.st_mode) or st.st_uid != os.getuid() or st.st_mode & 0o077:
+        raise RuntimeError('%s is not a private directory of this user: refusing to load libraries from it' % d)
+    return d
+
+
+def variant_tag(keys):
+    """Content hash of everything a model-specific library is built from: its tile structures, the kernel sources,
+    the build script and the compiler with its options.  Checkouts of different commits never share a library."""
+    h = hashlib.sha256()
+    for part in ['\n'.join(keys), _build.nvcc_path(), ' '.join(_build.NVCC_FLAGS)]:
+        h.update(part.encode() + b'\0')
+    for f in [os.path.join(_build.CSRC, d) for d in _build.DEPS] + [_build.__file__]:
+        with open(f, 'rb') as src:
+            h.update(src.read() + b'\0')
+    return h.hexdigest()[:16]
+
+
 def library_for(problem, verbose=False):
     """Path of a library whose kernel instances cover every tile structure of `problem`; builds it with nvcc when
     the stock library does not (returns None if nothing is needed, or if nvcc is missing)."""
@@ -82,15 +111,17 @@ def library_for(problem, verbose=False):
     except RuntimeError:
         return None
     keys = sorted(need | have)
-    tag = hashlib.sha1('\n'.join(keys).encode()).hexdigest()[:12]
-    lib = os.path.join(_build.LIBDIR, 'libmali_b200_spec_%s.so' % tag)
-    newest = max(os.path.getmtime(os.path.join(_build.CSRC, d)) for d in _build.DEPS if d != 'spec_instances.inc')
-    if os.path.isfile(lib) and os.path.getmtime(lib) >= newest:      # cached and not older than any kernel source
-        return lib
-    inc = os.path.join(_build.LIBDIR, 'spec_instances_%s.inc' % tag)
-    os.makedirs(_build.LIBDIR, exist_ok=True)
-    write_instances(keys, inc, '(stock + model-specific)')
-    if verbose:
-        sys.stderr.write('lightspinner_b200: building %s for %d new tile structures\n'
-                         % (os.path.basename(lib), len(need - have)))
-    return _build.build(force=True, verbose=False, lib=lib, spec_inc=inc)
+    tag = variant_tag(keys)
+    cache = cache_dir()
+    lib = os.path.join(cache, 'libmali_b200_spec_%s.so' % tag)
+    with open(lib + '.lock', 'w') as lock:      # the ranks of one job ask for the same library at the same time
+        fcntl.flock(lock, fcntl.LOCK_EX)
+        if os.path.isfile(lib):                 # the name is the hash of all its inputs; build() writes it atomically
+            return lib
+        inc = os.path.join(cache, 'spec_instances_%s.inc' % tag)
+        write_instances(keys, inc, '(stock + model-specific)')
+        if verbose:
+            sys.stderr.write('lightspinner_b200: building %s for %d new tile structures\n'
+                             % (os.path.basename(lib), len(need - have)))
+        return _build.build(force=True, verbose=False, lib=lib, spec_inc=inc,
+                            objdir=os.path.join(cache, '_obj', os.path.basename(lib)))

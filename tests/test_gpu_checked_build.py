@@ -1,7 +1,6 @@
-"""Stand-in for compute-sanitizer's racecheck on the TMA-ring protocol (the tool is closed on this pool,
-profiles/r02_sanitizer_closed.txt): the CHECKED build of the library (-DMALI_CHECK, tools/build_variants.py
-check:MALI_CHECK=1 -> lightspinner_b200/_lib/libmali_b200_check.so) makes every lane compare, at every depth step, what
-arrived through the ring -- heights, populations, background field, line-profile row -- with a direct global load of the
+"""Stand-in for compute-sanitizer's racecheck on the TMA-ring protocol: the CHECKED build of the library (-DMALI_CHECK,
+lightspinner_b200/_lib/libmali_b200_check.so, built next to the stock library by build()) makes every lane compare,
+at every depth step, what arrived through the ring -- heights, populations, background field, line-profile row -- with a direct global load of the
 same element of (tile, depth k), and raise status bit 2 (value 4) on any mismatch.  A ring stage refilled before its
 last reader was done, or read before its copy landed, cannot pass this: the stage would hold another depth's record.
 Run on every fixture shape (82 / 81 / 512 depths, 3 / 5 / 10 rays), both arithmetic modes, the per-call entry point and
@@ -13,17 +12,15 @@ import pytest
 import torch
 
 from helpers import drop_depth, load_golden
+from lightspinner_b200.build import CHECK_LIB as LIB
 
 pytestmark = pytest.mark.gpu
-LIB = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), 'lightspinner_b200', '_lib',
-                   'libmali_b200_check.so')
 
 
 @pytest.mark.parametrize('arith', ['exact', 'contracted'])
 @pytest.mark.parametrize('name', ['c1_falc_ca', 'c2_falc_cah', 'c1v_jitter_ca3', 'stress_r10_d512', 'c1_odd'])
 def test_ring_delivers_the_right_record_at_every_step(name, arith):
-    if not os.path.isfile(LIB):
-        pytest.skip('checked build not present (python tools/build_variants.py check:MALI_CHECK=1)')
+    assert os.path.isfile(LIB), 'checked build missing: __graft_entry__.build() makes it'
     from lightspinner_b200.engine import MaliEngine
     p, _ = load_golden('c1_falc_ca' if name == 'c1_odd' else name)
     if name == 'c1_odd':

@@ -55,24 +55,60 @@ def test_synthetic_jitter_is_deterministic_and_mild():
     assert np.all(np.abs(np.log(a['bg_chi'] / p['bg_chi'])) < 0.25)
 
 
-@pytest.mark.reference
+def _recorded_reference_objects(p):
+    """fake_reference_objects(p) whose model objects check each call the drop-in makes against the call the
+    reference's Context made when the fixture was recorded (tests/golden/make_golden.py stores its hGround, the
+    atoms' Doppler widths and LTE populations): v_broad, damping and compute_rates are asked with the
+    nondimensionalised atmosphere, damping with the atom's vBroad and the H ground population, compute_rates with the
+    atom's nStar and a zeroed C [Nlevel, Nlevel, Nspace].  Each is asked once per model object."""
+    atmos, spect, eqPops, bg = fake_reference_objects(p)
+    N = int(p['Nspace'])
+    lvloff = np.concatenate([[0], np.cumsum(p['Nlevel'])]).astype(int)
+    calls = []
+
+    def v_broad(at, atom):
+        assert at is atmos and not at.dimensioned
+        calls.append(('v_broad', atom.name))
+        return atom._vBroad
+
+    def damping(at, vBroad, hGround, line, atom):
+        assert at is atmos and not at.dimensioned
+        assert np.array_equal(vBroad, atom._vBroad) and np.array_equal(hGround, p['hGround'])
+        calls.append(('damping', id(line)))
+        return line._aDamp, None
+
+    def compute_rates(at, nStar, C, coll, a):
+        assert at is atmos and not at.dimensioned
+        NL = int(p['Nlevel'][a])
+        assert np.array_equal(nStar, p['nStar'][lvloff[a]:lvloff[a + 1]])
+        assert C.shape == (NL, NL, N) and not C.any()
+        calls.append(('compute_rates', a))
+        C += coll._C
+
+    for a, atom in enumerate(spect.radSet.activeAtoms):
+        atom.v_broad = lambda at, atom=atom: v_broad(at, atom)
+        for line in atom.lines:
+            line.damping = lambda at, vB, hG, line=line, atom=atom: damping(at, vB, hG, line, atom)
+        for coll in atom.collisions:
+            coll.compute_rates = lambda at, nStar, C, coll=coll, a=a: compute_rates(at, nStar, C, coll, a)
+    return (atmos, spect, eqPops, bg), calls
+
+
 def test_context_host_mirror_against_live_reference():
-    """With /root/reference present: the drop-in fed the REAL reference objects flattens to exactly what the
-    reference's own Context holds (C, Nblue, damping parameters, ...)."""
-    from oracle.refharness import reference_available, load_reference, build_falc_setup
-    if not reference_available():
-        pytest.skip('Lightspinner reference not present')
-    from oracle.refharness.extract import problem_from_reference_context
+    """The drop-in fed stand-ins of the reference's model objects that answer, and expect, what the reference's own
+    objects answered and were asked when the fixtures were recorded: it must ask each object the same question and
+    flatten the answers to exactly what the reference's Context held (C, Nblue, damping parameters, ...)."""
     from lightspinner_b200.context import Context
-    import copy
-    ref = load_reference()
-    atmos, spect, eqPops, bg = build_falc_setup(active=('Ca',), nrays=3)
-    eq2 = copy.deepcopy(eqPops)
-    rctx = ref['rh_method'].Context(atmos, spect, eqPops, bg)
-    pr = problem_from_reference_context(rctx)
-    ctx = Context(atmos, spect, eq2, bg, _host_only=True)
-    for k in KEYS:
-        assert np.array_equal(np.asarray(ctx._problem[k]), np.asarray(pr[k])), k
+    for name in ['c1_falc_ca', 'c2_falc_cah', 'c1v_jitter_ca3', 'rf_k40p']:
+        p, _ = load_golden(name)
+        (atmos, spect, eqPops, bg), calls = _recorded_reference_objects(p)
+        ctx = Context(atmos, spect, eqPops, bg, _host_only=True)
+        natom = len(p['Nlevel'])
+        nline = int(np.asarray(p['trans'])[:, 3].sum())
+        assert sorted(c[0] for c in calls) == sorted(['v_broad'] * natom + ['damping'] * nline + ['compute_rates'] * natom)
+        assert len(set(calls)) == len(calls), name
+        for k in KEYS:
+            assert np.array_equal(np.asarray(ctx._problem[k]), np.asarray(p[k])), (name, k)
 
 
 def test_stock_kernel_instances_cover_the_fixture_models():
@@ -98,35 +134,47 @@ def test_batch_context_rejects_columns_of_different_models():
         BatchContext([])
 
 
-@pytest.mark.reference
 def test_atom_and_eos_tables_from_live_reference_objects():
-    """With /root/reference present: the model-level tables of the device-side set-up built from the REAL reference
-    objects (AtomTables.from_models, EosTables.from_witt) equal the ones built from the committed fixtures
-    (tests/golden/setup_inputs.npz, eos.npz) -- the path a user of the reference takes and the path the GPU tests take
-    are the same data."""
-    from oracle.refharness import reference_available, load_reference
-    if not reference_available():
-        pytest.skip('Lightspinner reference not present')
+    """The model-level tables of the device-side set-up built from stand-ins of the reference's objects
+    (AtomTables.from_models: atomic models with levels and collision terms, and the atomic table; EosTables.from_witt:
+    a witt instance) equal the ones built from the committed fixtures (tests/golden/setup_inputs.npz, eos.npz) --
+    the path a user of the reference takes and the path the GPU tests take are the same data.  The stand-ins carry
+    the attributes the reference's objects held when the fixtures were recorded, under the reference's names."""
     import os
+    from types import SimpleNamespace as NS
     from helpers import GOLDEN, load_setup_inputs
     from lightspinner_b200.atoms import AtomTables
-    from lightspinner_b200.eos import EosTables
-    ref = load_reference()
-    models = [ref['rh_atoms'].H_6_atom(), ref['rh_atoms'].CaII_atom()]
-    table = ref['atomic_set'].RadiativeSet(models).atomicTable
-    live = AtomTables.from_models(models, table)
+    from lightspinner_b200.eos import NCONTR, EosTables
     atoms, _ = load_setup_inputs('c2_falc_cah')
+    kinds = [type(nm, (), {}) for nm in ('Omega', 'CI', 'CE')]     # collisional_rates.py's class names
+
+    def model(name, a):
+        levels = [NS(E_SI=e, g=g, stage=st) for e, g, st in zip(a['E_SI'], a['g'], a['stage'])]
+        colls, o = [], 0
+        for kind, i, j, n in a['coll']:
+            c = kinds[kind]()
+            c.i, c.j, c.temperature, c.rates = int(i), int(j), a['coll_T'][o:o + n], a['coll_rates'][o:o + n]
+            colls.append(c)
+            o += n
+        return NS(name=name, levels=levels, collisions=colls)
+
+    models = [model('H', atoms['H']), model('CA', atoms['CA'])]
+    table = {'H': NS(weight=atoms['H']['weight']), 'CA': NS(weight=atoms['CA']['weight'])}
+    live = AtomTables.from_models(models, table)
     fix = AtomTables.from_arrays([dict(atoms['H']), dict(atoms['CA'])])
     for k in ('Nlevel', 'dE', 'gi0', 'dZ', 'nDebye', 'g', 'vTherm', 'coll', 'knots', 'coef', 'fill', 'par'):
         assert np.array_equal(getattr(live, k), getattr(fix, k)), k
     assert live.c1 == fix.c1 and live.c2 == fix.c2
-    import witt as W
     z = np.load(os.path.join(GOLDEN, 'eos.npz'))
-    e_live = EosTables.from_witt(W.witt(), ref['atomic_table'].get_global_atomic_table().weightPerH)
+    off = z['stage_off']
+    el = [NS(pf=z['pf'][off[i]:off[i + 1]], eion=z['eion'][off[i]:off[i + 1]], nstage=int(off[i + 1] - off[i]))
+          for i in range(NCONTR)]
+    witt = NS(el=el, tpf=z['tpf'], ABUND=z['ABUND'], avw=float(z['avw']), rho_from_H=float(z['rho_from_H']),
+              ab_others=float(z['ab_others']), prec=1.e-5)
+    e_live = EosTables.from_witt(witt, float(z['weightPerH']))
     e_fix = EosTables.from_arrays(z)
     for k in ('tpf', 'pf', 'eion', 'stage_off'):
         assert np.array_equal(getattr(e_live, k), getattr(e_fix, k)), k
-    # witt.__init__ renormalises the class-level abundances in place on every instantiation: equal to rounding only
     assert np.allclose(e_live.abund, e_fix.abund, rtol=1e-14, atol=0)
     for k in ('avw', 'rho_from_H', 'ab_others', 'saha_fac', 'amu_wph', 'cm3', 'thomson'):
         assert abs(getattr(e_live, k) / getattr(e_fix, k) - 1.0) < 1e-14, k

@@ -31,8 +31,9 @@ def build_problem(refine=10, nrays=10, ndepth=512, base_name='stress_r10_d512'):
     return synth.stress_problem(base, refine=refine, nrays=nrays, ndepth=ndepth)
 
 
-def run(q, iters=6, init_dist=True):
-    """Times `iters` MALI iterations of the wavelength-sharded column on the ranks of the current torchrun launch.
+def run(q, iters=6, warmup=6, init_dist=True):
+    """Times `iters` MALI iterations of the wavelength-sharded column on the ranks of the current torchrun launch, after
+    a warm-up pass of `warmup` iterations (none when 0; each pass starts from fresh populations).
     Returns a dict (rank 0) with per-iteration times, split into formal solution / all-reduce / statistical equilibrium."""
     import torch
     import torch.distributed as dist
@@ -48,7 +49,7 @@ def run(q, iters=6, init_dist=True):
     info = col.eng.model_info()
     ev = lambda: torch.cuda.Event(enable_timing=True)
 
-    def one_pass():
+    def one_pass(iters):
         col.eng.upload([col.sub])
         col.eng.reset_iteration_state()
         torch.cuda.synchronize(dev)
@@ -72,8 +73,9 @@ def run(q, iters=6, init_dist=True):
             tot.append(e[0].elapsed_time(e[3]))
         return [float(np.median(x)) for x in (fs, ar, se, tot)]
 
-    one_pass()                                        # warm-up (library load, NCCL channels)
-    med = one_pass()
+    if warmup > 0:
+        one_pass(warmup)                              # warm-up (library load, NCCL channels)
+    med = one_pass(iters)
     ar_min = med[1]
     if world > 1:
         # the exchange segment of a rank includes its wait for the slowest rank's formal solution: the MIN over ranks (the
