@@ -16,6 +16,7 @@
  *   planck                      utils.py:17-22              mali_planck_bc (host helper for the lower boundary)
  *   Context.stat_equil          rh_method.py:710-745        mali_stat_equil
  *   test.py:20-29 / response_fn.py:11-21 (the MALI loop)    mali_iterate (device-resident loop, per-column convergence)
+ *   (no reference counterpart: opt-in Ng acceleration)      mali_stat_equil_ng, mali_iterate_ng; mali_ng_hook = test hook
  *   lte_pops atomic_set.py:105-145, compute_collisions rh_method.py:474-487, v_broad atomic_model.py:241-245,
  *   continuum g_ij rh_method.py:453-454                     mali_model_set_atoms + mali_setup_columns (device-side set-up)
  *   Background.compute_background_eos background.py:21-53 (witt.py EOS + cop), AtmosphereConstructor.convert_scales
@@ -259,6 +260,35 @@ int mali_stat_equil(const mali_model *m, const mali_buffers *bufs, int32_t col0,
 int mali_iterate(const mali_model *m, const mali_buffers *bufs, int32_t col0, int32_t ncol, int32_t max_iter,
                  double tolJ, double tolPops, void *stream);
 
+/* Ng acceleration of the population iteration (Auer 1987), opt-in; the reference has no such option, so with it on the
+ * iteration counts differ from the reference's.  Per column and active atom, the vector x = n[level][k] (flattened
+ * over level, depth) is pushed into a ring of the last order + 2 solved vectors after every statistical-equilibrium
+ * solve, and nse counts the column's solves since the caller last zeroed it.  When nse > delay, nse >= order + 2 and
+ * (nse - delay) % period == 0, with x0 the newest vector, d_i = x_i - x_{i+1} (i = 0..order) and w = 1/x0^2:
+ *     A_ij = sum w (d0 - d_{i+1})(d0 - d_{j+1}),  b_i = sum w d0 (d0 - d_{i+1}),  A c = b,
+ *     x* = (1 - sum c) x0 + sum_i c_i x_{i+1},
+ * accepted (replacing the populations and the newest ring entry) only if A is non-singular and every entry of x* is
+ * finite and > 0.  dPops of such an iteration is max |1 - n_start / n_final| over the column's atoms (n_start: what the
+ * solve started from).  1 <= order <= 3, delay >= 0, period >= 1 (else MALI_EINVAL); (2, 3, 3) is the measured default,
+ * (2, 2, 2) did not converge on CaII+H/FALC (DESIGN.md section 4).  The sums over (level, depth) are fixed-order block
+ * reductions: results do not depend on the batch or the column range. */
+typedef struct { int32_t order, delay, period; } mali_ng_params;
+typedef struct {
+    double *hist;      /* [ncol][mali_ng_layout doubles]: order+2 ring slots + 1 start snapshot, each sumNlevel*Nspace,
+                          then Natom doubles of library scratch */
+    int32_t *nse;      /* [ncol] solves since reset (caller zeroes; zero it again after editing a column's populations) */
+    int32_t *accepted; /* [ncol][Natom] extrapolations applied (caller zeroes) */
+} mali_ng_buffers;
+int mali_ng_layout(const mali_model *m, int32_t order, int64_t *doubles_per_column);
+/* mali_stat_equil followed by the Ng stage for columns [col0, col0+ncol). */
+int mali_stat_equil_ng(const mali_model *m, const mali_buffers *b, const mali_ng_buffers *ng, const mali_ng_params *p,
+                       int32_t col0, int32_t ncol, void *stream);
+/* mali_iterate with the Ng stage after every statistical equilibrium (same captured graph, cached per Ng buffers and
+ * parameters as well).  With delay >= max_iter no extrapolation is due and the results are bit-identical to
+ * mali_iterate's. */
+int mali_iterate_ng(const mali_model *m, const mali_buffers *b, const mali_ng_buffers *ng, const mali_ng_params *p,
+                    int32_t col0, int32_t ncol, int32_t max_iter, double tolJ, double tolPops, void *stream);
+
 /* Measurement: between begin and end every fs_gamma_kernel launch made through this model is bracketed by CUDA
  * events on its stream; end() returns their summed device time and the launch count (bench.py's roofline).
  * mali_launch_count: kernels launched through this model since creation (bench.py's gpu_launches). */
@@ -294,6 +324,9 @@ int mali_exp_hook(int32_t n, const double *x_dev, double *y_dev, void *stream);
 /* q[i] = a[i] / b[i] with the kernels' shared-reciprocal division; bad[i] != 0 where (a, b) is outside its domain.
  * Must equal the IEEE quotient bit for bit inside the domain. */
 int mali_div_hook(int32_t n, const double *a_dev, const double *b_dev, double *q_dev, int32_t *bad_dev, void *stream);
+/* One Ng extrapolation of hist_dev [order+2][nvec] (newest first) with the kernel's own code: out_dev = x* if accepted,
+ * else the newest vector; *accepted_dev = 1 / 0. */
+int mali_ng_hook(int32_t order, int64_t nvec, const double *hist_dev, double *out_dev, int32_t *accepted_dev, void *stream);
 /* ComputationalTransition.uv(la, mu, toFrom) for transition t of column col: writes Uji, Vij, Vji [Nspace]. */
 int mali_uv(const mali_model *m, const mali_buffers *bufs, int32_t col, int32_t t, int32_t la, int32_t mu,
             int32_t toFrom, double *Uji_dev, double *Vij_dev, double *Vji_dev, void *stream);

@@ -51,12 +51,21 @@ class Buffers(C.Structure):
                 ('dPops', C.c_void_p), ('status', C.c_void_p), ('iter', C.c_void_p), ('done', C.c_void_p)]
 
 
+class NgParams(C.Structure):
+    _fields_ = [('order', C.c_int32), ('delay', C.c_int32), ('period', C.c_int32)]
+
+
+class NgBuffers(C.Structure):
+    _fields_ = [('hist', C.c_void_p), ('nse', C.c_void_p), ('accepted', C.c_void_p)]
+
+
 EXPORTS = ['mali_last_error', 'mali_device_count', 'mali_model_create', 'mali_model_destroy', 'mali_model_layout', 'mali_model_info',
            'mali_planck_bc', 'mali_upload_columns', 'mali_upload_columns_nophi', 'mali_compute_phi', 'mali_formal_sol_gamma', 'mali_stat_equil', 'mali_iterate',
            'mali_piecewise_linear_1d', 'mali_uv', 'mali_exp_hook', 'mali_div_hook', 'mali_profile_begin',
            'mali_profile_end', 'mali_launch_count', 'mali_fp64_peak', 'mali_line_layout', 'mali_model_set_arith', 'mali_model_get_arith',
            'mali_upload_columns_atmos', 'mali_model_set_atoms', 'mali_setup_columns',
-           'mali_upload_columns_thermo', 'mali_model_set_eos', 'mali_background', 'mali_graph_iterations']
+           'mali_upload_columns_thermo', 'mali_model_set_eos', 'mali_background', 'mali_graph_iterations',
+           'mali_ng_layout', 'mali_stat_equil_ng', 'mali_iterate_ng', 'mali_ng_hook']
 
 ARITH_EXACT, ARITH_CONTRACTED = 0, 1
 
@@ -110,6 +119,12 @@ def load(path=None):
     L.mali_div_hook.argtypes = [C.c_int32] + [C.c_void_p] * 5
     L.mali_fp64_peak.argtypes = [C.c_int32, C.c_void_p, C.POINTER(C.c_double)]
     L.mali_exp_hook.argtypes = [C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p]
+    L.mali_ng_layout.argtypes = [C.c_void_p, C.c_int32, C.POINTER(C.c_int64)]
+    L.mali_stat_equil_ng.argtypes = [C.c_void_p, C.POINTER(Buffers), C.POINTER(NgBuffers), C.POINTER(NgParams), C.c_int32,
+                                     C.c_int32, C.c_void_p]
+    L.mali_iterate_ng.argtypes = [C.c_void_p, C.POINTER(Buffers), C.POINTER(NgBuffers), C.POINTER(NgParams), C.c_int32,
+                                  C.c_int32, C.c_int32, C.c_double, C.c_double, C.c_void_p]
+    L.mali_ng_hook.argtypes = [C.c_int32, C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
     L.mali_uv.argtypes = [C.c_void_p, C.POINTER(Buffers)] + [C.c_int32] * 5 + [C.c_void_p] * 4
     _libs[path] = L
     return L

@@ -146,10 +146,12 @@ class Context:
     same kernels over many columns per launch.
     """
 
-    def __init__(self, atmos, spect, eqPops, background, device=None, _host_only=False):
+    def __init__(self, atmos, spect, eqPops, background, device=None, ng=None, _host_only=False):
         """The Voigt line profiles (ComputationalTransition.compute_phi, rh_method.py:198-243) are formed on the GPU
         from the damping parameters -- same values to ~1e-13 (the accuracy of the scipy wofz the reference calls);
-        `trans.phi` / `trans.wphi` are read back from the device if somebody asks for them."""
+        `trans.phi` / `trans.wphi` are read back from the device if somebody asks for them.
+        ng: an NgOptions to accelerate the population iteration of stat_equil() (off by default; the reference has no
+        such option, so with it on the iteration count differs from the reference's)."""
         self.atmos = atmos
         self.atmos.nondimensionalise()                                    # rh_method.py:553
         self.spect = spect
@@ -164,7 +166,7 @@ class Context:
         self._col = 0       # column of the engine's batch this Context owns (BatchContext hands out others)
         if _host_only:      # unit tests of the host-side flattening only; every compute method then fails
             return
-        self._engine = MaliEngine(self._problem, 1, device=device)
+        self._engine = MaliEngine(self._problem, 1, device=device, ng=ng)
         self._engine.upload_device_phi([self._problem])
 
     # -- lazily fetched results (numpy, C order, the reference's shapes)
@@ -200,6 +202,10 @@ class Context:
         self._pull_pops()
         return dPops
 
+    def ng_reset(self):
+        """Restart the Ng history (Context(ng=...)): call it after editing populations between iterations."""
+        self._engine.ng_reset(self._col, 1)
+
     def _pull_pops(self):
         n = self._engine.n(self._col)
         mt = self._engine.mt
@@ -224,7 +230,8 @@ class BatchContext:
     methods of the reference exist in batched form too: formal_sol_gamma_matrices() and stat_equil() return one
     value per column."""
 
-    def __init__(self, columns, device=None):
+    def __init__(self, columns, device=None, ng=None):
+        """ng: an NgOptions to accelerate the population iteration (off by default, see Context)."""
         if not columns:
             raise ValueError('BatchContext needs at least one column')
         self.contexts = [Context(*c, _host_only=True) for c in columns]
@@ -237,7 +244,7 @@ class BatchContext:
             for key in ('trans', 'wavelength', 'muz', 'wmu', 'Nlevel', 'linepar', 'alpha'):
                 if not np.array_equal(np.asarray(q[key]), np.asarray(p0[key])):
                     raise ValueError('columns of a batch must share the radiative model (%s differs)' % key)
-        self._engine = MaliEngine(p0, len(problems), device=device)
+        self._engine = MaliEngine(p0, len(problems), device=device, ng=ng)
         self._engine.upload_device_phi(problems)
         for k, c in enumerate(self.contexts):
             c._engine, c._col, c._borrowed = self._engine, k, True

@@ -55,8 +55,9 @@ cudaError_t to_device(const std::vector<T> &h, T **d)
 
 // First kernel of every statistical-equilibrium stage: inside mali_iterate it counts the iteration (test.py:24;
 // the formal solution of this iteration is done), then resets dPops of the columns that are about to be solved.
+// With Ng acceleration (nse != null) it also counts the solve in the column's nse.
 __global__ void se_prepare_kernel(unsigned long long *bits, const int32_t *done, int32_t *iter, int iterMin, int count,
-                                  int col0, int ncol)
+                                  int col0, int ncol, int32_t *nse)
 {
     const int c = blockIdx.x * blockDim.x + threadIdx.x;
     if (c >= ncol) return;
@@ -67,6 +68,7 @@ __global__ void se_prepare_kernel(unsigned long long *bits, const int32_t *done,
         if (iter[col] < iterMin) return;
     }
     bits[col] = 0ull;
+    if (nse != nullptr) nse[col] += 1;
 }
 
 // First kernel of every formal solution, one block per column: resets dJ and rebuilds the depth-major popsT table
@@ -145,6 +147,8 @@ struct IterGraphKey {
     int32_t col0, ncol;
     double tolJ, tolPops;
     int32_t arith;
+    mali_ng_buffers ng;      // all zero for mali_iterate: a plain graph is never replayed for an Ng call, or the reverse
+    mali_ng_params ngp;
 };
 struct IterGraph {
     IterGraphKey key;
@@ -1245,21 +1249,77 @@ static int launch_fs(const mali_model *m, const mali_buffers *b, int col0, int n
     return MALI_OK;
 }
 
+static int64_t ng_doubles_per_column(const mali_model *m, int order)
+{
+    // order + 2 ring slots and the start snapshot, each [sumNlevel][Nspace], then one dPops bit pattern per atom
+    return (int64_t)(order + 3) * m->lay.pops + m->Natom;
+}
+
+// ng != null: the statistical equilibrium also counts the solve (nse), snapshots n and pushes the solution into the
+// ring, and the Ng stage follows it (ng_kernel, ng_dpops_kernel).  Without ng the launches are those of before.
 static int launch_se(const mali_model *m, const mali_buffers *b, int col0, int ncol, int32_t *iter, int iterMin,
-                     cudaStream_t st)
+                     cudaStream_t st, const mali_ng_buffers *ng = nullptr, const mali_ng_params *ngp = nullptr)
 {
     FinishParams f = make_finish_params(m, b, col0, ncol);
     // inside mali_iterate, columns whose own iteration counter is still <= 3 only iterate J (test.py:27)
     f.iter = iter;
     f.iterMin = iterMin;
-    se_prepare_kernel<<<(ncol + 127) / 128, 128, 0, st>>>(f.dPopsBits, b->done, iter, iterMin, iter != nullptr, col0, ncol);
+    if (ng) {
+        f.ngHist = ng->hist;
+        f.ngNse = ng->nse;
+        f.ngStride = ng_doubles_per_column(m, ngp->order);
+        f.ngRing = ngp->order + 2;
+    }
+    se_prepare_kernel<<<(ncol + 127) / 128, 128, 0, st>>>(f.dPopsBits, b->done, iter, iterMin, iter != nullptr, col0, ncol,
+                                                          ng ? ng->nse : nullptr);
     dim3 grid((m->N + 63) / 64, m->Natom, ncol);
     if (m->maxNlevel <= 8)
         stat_equil_kernel<8><<<grid, 64, 0, st>>>(f);
     else
         stat_equil_kernel<16><<<grid, 64, 0, st>>>(f);
     m->launches += 2;
+    if (ng) {
+        NgParams q{};
+        q.N = m->N;
+        q.Natom = m->Natom;
+        q.col0 = col0;
+        q.order = ngp->order;
+        q.delay = ngp->delay;
+        q.period = ngp->period;
+        q.ring = ngp->order + 2;
+        q.iterMin = iterMin;
+        q.popStride = m->lay.pops;
+        q.histStride = f.ngStride;
+        q.Nlevel = m->d_Nlevel;
+        q.lvlOff = m->d_lvlOff;
+        q.pops = b->pops;
+        q.hist = ng->hist;
+        q.nse = ng->nse;
+        q.accepted = ng->accepted;
+        q.dPops = b->dPops;
+        q.status = b->status;
+        q.done = b->done;
+        q.iter = iter;
+        dim3 g(m->Natom, ncol);
+        if (q.order == 1)
+            ng_kernel<1><<<g, kNgThreads, 0, st>>>(q);
+        else if (q.order == 2)
+            ng_kernel<2><<<g, kNgThreads, 0, st>>>(q);
+        else
+            ng_kernel<3><<<g, kNgThreads, 0, st>>>(q);
+        ng_dpops_kernel<<<(ncol + 127) / 128, 128, 0, st>>>(q, ncol);
+        m->launches += 2;
+    }
     CU(cudaGetLastError());
+    return MALI_OK;
+}
+
+static int check_ng(const mali_ng_buffers *ng, const mali_ng_params *p, const char *who)
+{
+    if (!ng || !p || !ng->hist || !ng->nse || !ng->accepted) return fail(MALI_EINVAL, "%s: null Ng buffer or parameters", who);
+    if (p->order < 1 || p->order > 3 || p->delay < 0 || p->period < 1)
+        return fail(MALI_EINVAL, "%s: Ng order=%d delay=%d period=%d (need 1 <= order <= 3, delay >= 0, period >= 1)", who,
+                    p->order, p->delay, p->period);
     return MALI_OK;
 }
 
@@ -1286,8 +1346,46 @@ int mali_stat_equil(const mali_model *m, const mali_buffers *b, int32_t col0, in
     return launch_se(m, &bb, col0, ncol, nullptr, 0, (cudaStream_t)stream);
 }
 
+int mali_ng_layout(const mali_model *m, int32_t order, int64_t *doubles_per_column)
+{
+    if (!m || !doubles_per_column || order < 1 || order > 3) return fail(MALI_EINVAL, "mali_ng_layout: bad argument (order %d)", order);
+    *doubles_per_column = ng_doubles_per_column(m, order);
+    return MALI_OK;
+}
+
+int mali_stat_equil_ng(const mali_model *m, const mali_buffers *b, const mali_ng_buffers *ng, const mali_ng_params *p,
+                       int32_t col0, int32_t ncol, void *stream)
+{
+    if (int r = check_range(m, b, col0, ncol, "mali_stat_equil_ng")) return r;
+    if (int r = check_ng(ng, p, "mali_stat_equil_ng")) return r;
+    if (!b->colconst || !b->pops || !b->Gamma || !b->dPops || !b->status)
+        return fail(MALI_EINVAL, "mali_stat_equil_ng: null buffer");
+    mali_buffers bb = *b;
+    bb.done = nullptr;
+    bb.iter = nullptr;
+    return launch_se(m, &bb, col0, ncol, nullptr, 0, (cudaStream_t)stream, ng, p);
+}
+
+static int iterate_impl(const mali_model *m, const mali_buffers *b, int32_t col0, int32_t ncol, int32_t max_iter,
+                        double tolJ, double tolPops, void *stream, const mali_ng_buffers *ng, const mali_ng_params *ngp);
+
 int mali_iterate(const mali_model *m, const mali_buffers *b, int32_t col0, int32_t ncol, int32_t max_iter, double tolJ,
                  double tolPops, void *stream)
+{
+    return iterate_impl(m, b, col0, ncol, max_iter, tolJ, tolPops, stream, nullptr, nullptr);
+}
+
+int mali_iterate_ng(const mali_model *m, const mali_buffers *b, const mali_ng_buffers *ng, const mali_ng_params *p,
+                    int32_t col0, int32_t ncol, int32_t max_iter, double tolJ, double tolPops, void *stream)
+{
+    if (int r = check_range(m, b, col0, ncol, "mali_iterate_ng")) return r;
+    if (int r = check_ng(ng, p, "mali_iterate_ng")) return r;
+    return iterate_impl(m, b, col0, ncol, max_iter, tolJ, tolPops, stream, ng, p);
+}
+
+// mali_iterate, and with ng: the Ng stage after every statistical equilibrium, inside the same captured graph
+static int iterate_impl(const mali_model *m, const mali_buffers *b, int32_t col0, int32_t ncol, int32_t max_iter,
+                        double tolJ, double tolPops, void *stream, const mali_ng_buffers *ng, const mali_ng_params *ngp)
 {
     if (int r = check_range(m, b, col0, ncol, "mali_iterate")) return r;
     if (!b->colconst || !b->pops || !b->J || !b->I || !b->Gamma || !b->scratch || !b->dJ || !b->dPops || !b->status ||
@@ -1317,7 +1415,7 @@ int mali_iterate(const mali_model *m, const mali_buffers *b, int32_t col0, int32
     auto one_iteration = [&]() -> int {
         bool jJoin = false;
         if (int r = launch_fs(m, b, col0, ncol, st, ctl, &jJoin)) return r;
-        if (int r = launch_se(m, b, col0, ncol, b->iter, 4, st)) return r;
+        if (int r = launch_se(m, b, col0, ncol, b->iter, 4, st, ng, ngp)) return r;
         if (jJoin) CU(cudaStreamWaitEvent(st, m->joinEvent[0], 0));
         return MALI_OK;
     };
@@ -1346,6 +1444,14 @@ int mali_iterate(const mali_model *m, const mali_buffers *b, int32_t col0, int32
         key.tolJ = tolJ;
         key.tolPops = tolPops;
         key.arith = m->arith;
+        if (ng) {
+            key.ng.hist = ng->hist;
+            key.ng.nse = ng->nse;
+            key.ng.accepted = ng->accepted;
+            key.ngp.order = ngp->order;
+            key.ngp.delay = ngp->delay;
+            key.ngp.period = ngp->period;
+        }
         cudaGraphExec_t exec = nullptr;
         for (auto &g : m->iterGraphs)
             if (memcmp(&g.key, &key, sizeof key) == 0) exec = g.exec;
@@ -1487,6 +1593,21 @@ int mali_fp64_peak(int32_t iters, double *scratch_dev, double *ops_per_second)
     CU(cudaEventDestroy(e0));
     CU(cudaEventDestroy(e1));
     *ops_per_second = (double)blocks * threads * (double)iters * 16.0 / (ms * 1e-3);  // 8 chains x (mul + add)
+    return MALI_OK;
+}
+
+int mali_ng_hook(int32_t order, int64_t nvec, const double *hist_dev, double *out_dev, int32_t *accepted_dev, void *stream)
+{
+    if (order < 1 || order > 3 || nvec < 1 || !hist_dev || !out_dev || !accepted_dev)
+        return fail(MALI_EINVAL, "mali_ng_hook: bad argument");
+    cudaStream_t st = (cudaStream_t)stream;
+    if (order == 1)
+        ng_hook_kernel<1><<<1, kNgThreads, 0, st>>>(nvec, hist_dev, out_dev, accepted_dev);
+    else if (order == 2)
+        ng_hook_kernel<2><<<1, kNgThreads, 0, st>>>(nvec, hist_dev, out_dev, accepted_dev);
+    else
+        ng_hook_kernel<3><<<1, kNgThreads, 0, st>>>(nvec, hist_dev, out_dev, accepted_dev);
+    CU(cudaGetLastError());
     return MALI_OK;
 }
 

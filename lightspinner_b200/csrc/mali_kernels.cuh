@@ -352,6 +352,12 @@ __global__ void stat_equil_kernel(const FinishParams p)
             iEl = l;
         }
     }
+    double *ngH = nullptr;   // Ng acceleration: this column's history block, shifted to this atom's first level
+    if (p.ngHist != nullptr) {
+        ngH = p.ngHist + (size_t)col * p.ngStride + (size_t)p.lvlOff[a] * N + k;
+        double *snap = ngH + (size_t)p.ngRing * p.popStride;   // n as the solve found it (dPops of an extrapolation)
+        for (int l = 0; l < NL; ++l) snap[(size_t)l * N] = n[(size_t)l * N + k];
+    }
     double x[NLMAX];
     if (!solve_stat_equil_any<NLMAX>(G, N, NL, iEl, nTot, x)) {
         atomicOr(p.status + col, 1);  // the reference would raise LinAlgError here
@@ -364,7 +370,234 @@ __global__ void stat_equil_kernel(const FinishParams p)
         db = b > db ? b : db;
         n[(size_t)l * N + k] = x[l];
     }
+    if (ngH != nullptr) {    // push the solution into the ring (the newest slot; ngNse already counts this solve)
+        double *slot = ngH + (size_t)((p.ngNse[col] - 1) % p.ngRing) * p.popStride;
+        for (int l = 0; l < NL; ++l) slot[(size_t)l * N] = x[l];
+    }
     atomicMax(p.dPopsBits + col, db);
+}
+
+// --------------------------------------------------------------------------------------------------------
+// Ng acceleration of the population iteration (Auer 1987), per column and active atom.  The vector is the atom's
+// populations x = n[level][k] flattened over (level, depth); x0 is the newest solved vector, x1, x2, ... the older
+// ones.  With d_i = x_i - x_{i+1} (i = 0..order) and w = 1 / x0^2 elementwise, solve the order x order system
+//     A c = b,   A_ij = sum w (d0 - d_{i+1})(d0 - d_{j+1}),   b_i = sum w d0 (d0 - d_{i+1}),
+// and form x* = (1 - sum c) x0 + sum_i c_i x_{i+1}.  x* is accepted only if A is non-singular and every entry of x* is
+// finite and > 0.  The sums are block-wide: a fixed element-to-thread assignment, a warp shuffle tree, then the
+// warps' sums added in warp order -- no atomics, so the result does not depend on the batch or the column range.
+// ng_solve_block is shared by ng_kernel and the test hook (mali_ng_hook).
+constexpr int kNgThreads = 256;
+
+__host__ __device__ __forceinline__ bool ng_due(int nse, int order, int delay, int period)
+{
+    return nse > delay && nse >= order + 2 && (nse - delay) % period == 0;
+}
+
+template <int ORDER>
+__device__ __forceinline__ double ng_value(const double *const *x, const double *c, double keep, int64_t idx)
+{
+    double v = keep * x[0][idx];
+#pragma unroll
+    for (int i = 0; i < ORDER; ++i) v = v + c[i] * x[i + 1][idx];
+    return v;
+}
+
+// Block-wide (kNgThreads threads, every one of them must call it): the coefficients c[ORDER] and 1 - sum c of the
+// extrapolation of the vectors x[0..ORDER+1] (length n), and whether x* is accepted.  The result is block-uniform.
+template <int ORDER>
+__device__ bool ng_solve_block(const double *const *x, int64_t n, double *c, double *keep)
+{
+    constexpr int kA = ORDER * (ORDER + 1) / 2, kS = kA + ORDER;   // upper triangle of A, then b
+    __shared__ double wsum[kNgThreads / 32][kS];
+    double s[kS];
+#pragma unroll
+    for (int q = 0; q < kS; ++q) s[q] = 0.0;
+    for (int64_t idx = threadIdx.x; idx < n; idx += kNgThreads) {
+        double d[ORDER + 1], e[ORDER];
+#pragma unroll
+        for (int i = 0; i <= ORDER; ++i) d[i] = x[i][idx] - x[i + 1][idx];
+        const double x0 = x[0][idx];
+        const double w = 1.0 / (x0 * x0);
+#pragma unroll
+        for (int i = 0; i < ORDER; ++i) e[i] = d[0] - d[i + 1];
+        int q = 0;
+#pragma unroll
+        for (int i = 0; i < ORDER; ++i) {
+            const double we = w * e[i];
+#pragma unroll
+            for (int j = i; j < ORDER; ++j) s[q++] += we * e[j];
+        }
+        const double wd = w * d[0];
+#pragma unroll
+        for (int i = 0; i < ORDER; ++i) s[kA + i] += wd * e[i];
+    }
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+#pragma unroll
+    for (int q = 0; q < kS; ++q) {
+        double v = s[q];
+#pragma unroll
+        for (int off = 16; off > 0; off >>= 1) v += __shfl_down_sync(0xffffffffu, v, off);
+        if (lane == 0) wsum[warp][q] = v;
+    }
+    __syncthreads();
+    // every thread adds the warps' sums in the same order and solves the same small system: no broadcast needed
+    double M[ORDER][ORDER + 1];
+    {
+        double t[kS];
+#pragma unroll
+        for (int q = 0; q < kS; ++q) {
+            t[q] = wsum[0][q];
+            for (int w = 1; w < kNgThreads / 32; ++w) t[q] += wsum[w][q];
+        }
+        int q = 0;
+#pragma unroll
+        for (int i = 0; i < ORDER; ++i)
+#pragma unroll
+            for (int j = i; j < ORDER; ++j) {
+                M[i][j] = t[q];
+                M[j][i] = t[q];
+                ++q;
+            }
+#pragma unroll
+        for (int i = 0; i < ORDER; ++i) M[i][ORDER] = t[kA + i];
+    }
+    // Gaussian elimination with partial pivoting; an exactly zero (or non-finite) pivot is a singular system
+    bool ok = true;
+#pragma unroll
+    for (int col = 0; col < ORDER; ++col) {
+        int piv = col;
+#pragma unroll
+        for (int r = col + 1; r < ORDER; ++r)
+            if (fabs(M[r][col]) > fabs(M[piv][col])) piv = r;
+        if (piv != col)
+#pragma unroll
+            for (int j = 0; j <= ORDER; ++j) {
+                const double tmp = M[col][j];
+                M[col][j] = M[piv][j];
+                M[piv][j] = tmp;
+            }
+        const double pv = M[col][col];
+        if (!(fabs(pv) > 0.0) || !isfinite(pv)) ok = false;
+#pragma unroll
+        for (int r = col + 1; r < ORDER; ++r) {
+            const double f = M[r][col] / pv;
+#pragma unroll
+            for (int j = col; j <= ORDER; ++j) M[r][j] = M[r][j] - f * M[col][j];
+        }
+    }
+    double csum = 0.0;
+#pragma unroll
+    for (int i = ORDER - 1; i >= 0; --i) {
+        double v = M[i][ORDER];
+#pragma unroll
+        for (int j = i + 1; j < ORDER; ++j) v = v - M[i][j] * c[j];
+        c[i] = v / M[i][i];
+    }
+#pragma unroll
+    for (int i = 0; i < ORDER; ++i) {
+        csum = csum + c[i];
+        if (!isfinite(c[i])) ok = false;
+    }
+    *keep = 1.0 - csum;
+    // positivity / finiteness vote over every entry of x*
+    bool good = ok;
+    if (ok)
+        for (int64_t idx = threadIdx.x; idx < n; idx += kNgThreads) {
+            const double v = ng_value<ORDER>(x, c, *keep, idx);
+            good = good && v > 0.0 && isfinite(v);
+        }
+    return __syncthreads_and(good) != 0;
+}
+
+struct NgParams {
+    int32_t N, Natom, col0, order, delay, period, ring, iterMin;
+    int64_t popStride, histStride;
+    const int32_t *Nlevel, *lvlOff;
+    double *pops, *hist;           // hist: per column ring slots, the snapshot, then one dPops bit pattern per atom
+    int32_t *nse, *accepted;       // [ncol], [ncol][Natom]
+    double *dPops;
+    const int32_t *status, *done, *iter;   // done / iter may be null (per-call entry point)
+};
+
+__device__ __forceinline__ bool ng_column_active(const NgParams &p, int col)
+{
+    if (p.done != nullptr && p.done[col] != 0) return false;        // as stat_equil_kernel: not solved this iteration
+    if (p.iter != nullptr && p.iter[col] < p.iterMin) return false;
+    if (p.status[col] != 0) return false;                           // a singular system: the column is failing
+    return ng_due(p.nse[col], p.order, p.delay, p.period);
+}
+
+// One block per (atom, column): the extrapolation, the write-back into n and the newest ring slot, and the atom's
+// max |1 - n_start / n_final| (bit pattern, combined over the atoms by ng_dpops_kernel).
+template <int ORDER>
+__global__ void __launch_bounds__(kNgThreads) ng_kernel(const NgParams p)
+{
+    const int a = blockIdx.x, col = p.col0 + blockIdx.y;
+    if (!ng_column_active(p, col)) return;
+    const int R = ORDER + 2, s = p.nse[col];
+    const int64_t off = (int64_t)p.lvlOff[a] * p.N, len = (int64_t)p.Nlevel[a] * p.N;
+    double *H = p.hist + (size_t)col * p.histStride;
+    const double *x[ORDER + 2];
+#pragma unroll
+    for (int i = 0; i < R; ++i) x[i] = H + (size_t)((s - 1 - i) % R) * p.popStride + off;
+    double c[ORDER], keep;
+    const bool acc = ng_solve_block<ORDER>(x, len, c, &keep);
+    double *n = p.pops + (size_t)col * p.popStride + off;
+    double *newest = H + (size_t)((s - 1) % R) * p.popStride + off;
+    const double *snap = H + (size_t)R * p.popStride + off;
+    unsigned long long db = 0ull;
+    for (int64_t idx = threadIdx.x; idx < len; idx += kNgThreads) {
+        double v = n[idx];
+        if (acc) {
+            v = ng_value<ORDER>(x, c, keep, idx);   // reads x0 = newest[idx] before this thread overwrites it
+            n[idx] = v;
+            newest[idx] = v;
+        }
+        const unsigned long long b = absbits(1.0 - snap[idx] / v);
+        db = b > db ? b : db;
+    }
+#pragma unroll
+    for (int off2 = 16; off2 > 0; off2 >>= 1) {
+        const unsigned long long o = __shfl_xor_sync(0xffffffffu, db, off2);
+        db = o > db ? o : db;
+    }
+    __shared__ unsigned long long wmax[kNgThreads / 32];
+    if ((threadIdx.x & 31) == 0) wmax[threadIdx.x >> 5] = db;
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        for (int w = 1; w < kNgThreads / 32; ++w) db = wmax[w] > db ? wmax[w] : db;
+        H[(size_t)(R + 1) * p.popStride + a] = __longlong_as_double((long long)db);
+        if (acc) p.accepted[(size_t)col * p.Natom + a] += 1;
+    }
+}
+
+// dPops of the iteration for the columns that were extrapolated: the max over the atoms, in atom order.
+__global__ void ng_dpops_kernel(const NgParams p, int ncol)
+{
+    const int c = blockIdx.x * blockDim.x + threadIdx.x;
+    if (c >= ncol) return;
+    const int col = p.col0 + c;
+    if (!ng_column_active(p, col)) return;
+    const double *part = p.hist + (size_t)col * p.histStride + (size_t)(p.ring + 1) * p.popStride;
+    unsigned long long db = 0ull;
+    for (int a = 0; a < p.Natom; ++a) {
+        const unsigned long long b = (unsigned long long)__double_as_longlong(part[a]);
+        db = b > db ? b : db;
+    }
+    p.dPops[col] = __longlong_as_double((long long)db);
+}
+
+// Test hook: one extrapolation of hist [ORDER+2][n] (newest first) -> out (x* if accepted, else x0).
+template <int ORDER>
+__global__ void __launch_bounds__(kNgThreads) ng_hook_kernel(int64_t n, const double *hist, double *out, int32_t *accepted)
+{
+    const double *x[ORDER + 2];
+#pragma unroll
+    for (int i = 0; i < ORDER + 2; ++i) x[i] = hist + (size_t)i * n;
+    double c[ORDER], keep;
+    const bool acc = ng_solve_block<ORDER>(x, n, c, &keep);
+    for (int64_t idx = threadIdx.x; idx < n; idx += kNgThreads) out[idx] = acc ? ng_value<ORDER>(x, c, keep, idx) : x[0][idx];
+    if (threadIdx.x == 0) *accepted = acc ? 1 : 0;
 }
 
 // --------------------------------------------------------------------------------------------------------

@@ -117,6 +117,13 @@ struct FinishParams {
     const int32_t *done;
     const int32_t *iter;  // may be null; with iter: only columns with iter[col] >= iterMin are solved
     int32_t iterMin;
+    // Ng acceleration (mali_stat_equil_ng / mali_iterate_ng; null otherwise): per column ngStride doubles holding
+    // ngRing ring slots of [sumNlevel][N] solved populations, then the snapshot of n taken before the solve.
+    // stat_equil_kernel writes the snapshot and pushes the solution into slot (ngNse[col] - 1) % ngRing.
+    double *ngHist;
+    const int32_t *ngNse;
+    int64_t ngStride;
+    int32_t ngRing;
 };
 
 }  // namespace mali

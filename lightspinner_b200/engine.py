@@ -20,14 +20,16 @@ from .tables import ModelTables, pack_column
 
 
 class MaliEngine:
-    def __init__(self, model, ncol, device=None, max_upload_chunk=64, specialize=False, arith=None, library=None):
+    def __init__(self, model, ncol, device=None, max_upload_chunk=64, specialize=False, arith=None, library=None, ng=None):
         """arith: 'exact' | 'contracted' | None (the library's default / the MALI_ARITH environment variable) -- the
         arithmetic mode of the formal-solution kernels, see include/mali_b200.h (mali_model_set_arith).
         library: path of another build of the library with the same ABI (e.g. the checked build of tools/build_variants.py).
         specialize=True: if the model has wavelength tiles without a specialised kernel instance and nvcc is
         available, build (once, cached) a model-specific variant of the library; otherwise those tiles run on the
         generic kernel.  specialize=<problem dict>: build / pick the variant that covers THAT model (e.g. the full
-        column when `model` is one wavelength shard of it, so that every rank loads the same library)."""
+        column when `model` is one wavelength shard of it, so that every rank loads the same library).
+        ng: an NgOptions to enable Ng acceleration of the population iteration (stat_equil, iterate_async); None: off,
+        and every launch and result is that of the plain iteration."""
         if not torch.cuda.is_available():
             raise RuntimeError('lightspinner_b200 needs a CUDA device: the MALI hot path has no CPU fallback')
         self.mt = model if isinstance(model, ModelTables) else ModelTables(model)
@@ -73,6 +75,18 @@ class MaliEngine:
         self.chunk = max(1, min(int(max_upload_chunk), n))
         self._staging = None
         self._pinned = None
+        self.ng = ng
+        if ng is not None:
+            from .ng import NgOptions
+            if not isinstance(ng, NgOptions):
+                raise TypeError('ng must be an NgOptions (or None)')
+            per = C.c_int64(0)
+            self._check(self.lib.mali_ng_layout(self._handle, ng.order, C.byref(per)))
+            self.t_ng_hist = torch.zeros(n * per.value, **f64)
+            self.t_ng_nse = torch.zeros(n, **i32)
+            self.t_ng_accepted = torch.zeros(n * self.mt.Natom, **i32)
+            self.ng_bufs = _capi.NgBuffers(*(t.data_ptr() for t in (self.t_ng_hist, self.t_ng_nse, self.t_ng_accepted)))
+            self.ng_params = _capi.NgParams(ng.order, ng.delay, ng.period)
 
     def _check(self, code):
         _capi.check(code, self.lib)
@@ -135,6 +149,7 @@ class MaliEngine:
         rh_method.py:198-243 -> mali_compute_phi) from each problem's damping parameters `aDamp` [Ntrans, Nspace],
         Doppler widths `vBroad` [Natom, Nspace] and `vlos` [Nspace]: only the blocks without phi / wphi (about 40 %
         of the bytes) cross PCIe.  Profiles agree with the reference's to ~1e-13 (the accuracy of scipy's wofz)."""
+        self.ng_reset(col0, len(problems))
         hpp = int(self.lay.hp_phi)
         staging, pinned = self._staging_bufs(hpp)
         pin_np = pinned.numpy()
@@ -169,6 +184,7 @@ class MaliEngine:
         lines' damping parameters aDamp; LTE populations, collisional rates, Doppler widths, the continua's g_ij
         (mali_setup_columns) and the Voigt profiles (mali_compute_phi) are computed on the GPU.  start_from_lte=False
         keeps the populations given in problem['n'] (a warm start, response_fn.py:33).  Needs set_atoms()."""
+        self.ng_reset(col0, len(problems))
         hpc = int(self.lay.hp_C)
         staging, pinned = self._staging_bufs(hpc)
         pin_np = pinned.numpy()
@@ -215,6 +231,7 @@ class MaliEngine:
         opacities (mali_background), LTE populations, collisional rates, Doppler widths, the continua's g_ij
         (mali_setup_columns) and the Voigt profiles (mali_compute_phi) are all formed on the GPU.
         Needs set_eos() and set_atoms()."""
+        self.ng_reset(col0, len(problems))
         hpb = int(self.lay.hp_bg_chi)
         staging, pinned = self._staging_bufs(hpb)
         pin_np = pinned.numpy()
@@ -255,6 +272,7 @@ class MaliEngine:
     def upload_packed_device_phi(self, host_prefix_pinned, aDamp, vBroad, vlos, col0, ncol, staging=None):
         """Asynchronous form of upload_device_phi: `host_prefix_pinned` holds [ncol][lay.hp_phi] doubles (pinned),
         aDamp / vBroad / vlos are device tensors [ncol][Ntrans|Natom|1][Nspace]."""
+        self.ng_reset(col0, ncol)
         if staging is None:
             staging, _ = self._staging_bufs(0)
         if ncol * self.lay.hostpack > staging.numel():
@@ -269,6 +287,7 @@ class MaliEngine:
 
     def upload_packed(self, host_pinned, col0, ncol, staging=None):
         """H2D copy of `ncol` host-pack blocks (a pinned torch tensor) + device re-layout; asynchronous."""
+        self.ng_reset(col0, ncol)
         if staging is None:
             staging, _ = self._staging_bufs(0)
         if ncol * self.lay.hostpack > staging.numel():
@@ -280,6 +299,7 @@ class MaliEngine:
 
     def repack_from_staging(self, staging, col0, ncol):
         """Device re-layout only (the staging tensor already holds host-pack blocks on the device)."""
+        self.ng_reset(col0, ncol)
         with torch.cuda.device(self.device):
             self._check(self.lib.mali_upload_columns(self._handle, C.byref(self.bufs), col0, ncol, None,
                                                      C.c_void_p(staging.data_ptr()), self._stream()))
@@ -293,7 +313,11 @@ class MaliEngine:
     def stat_equil_async(self, col0=0, ncol=None):
         ncol = self.ncol - col0 if ncol is None else ncol
         with torch.cuda.device(self.device):
-            self._check(self.lib.mali_stat_equil(self._handle, C.byref(self.bufs), col0, ncol, self._stream()))
+            if self.ng is not None:
+                self._check(self.lib.mali_stat_equil_ng(self._handle, C.byref(self.bufs), C.byref(self.ng_bufs),
+                                                        C.byref(self.ng_params), col0, ncol, self._stream()))
+            else:
+                self._check(self.lib.mali_stat_equil(self._handle, C.byref(self.bufs), col0, ncol, self._stream()))
 
     def formal_sol_gamma_matrices(self, col0=0, ncol=None):
         """One Lambda iteration for columns [col0, col0+ncol) (default: all); returns their dJ (device->host read)."""
@@ -324,8 +348,13 @@ class MaliEngine:
         """The loop of test.py:20-29 on the device with per-column convergence (tolJ < 0: fixed iteration count)."""
         ncol = self.ncol - col0 if ncol is None else ncol
         with torch.cuda.device(self.device):
-            self._check(self.lib.mali_iterate(self._handle, C.byref(self.bufs), col0, ncol, int(max_iter),
-                                              float(tolJ), float(tolPops), self._stream()))
+            if self.ng is not None:
+                self._check(self.lib.mali_iterate_ng(self._handle, C.byref(self.bufs), C.byref(self.ng_bufs),
+                                                     C.byref(self.ng_params), col0, ncol, int(max_iter), float(tolJ),
+                                                     float(tolPops), self._stream()))
+            else:
+                self._check(self.lib.mali_iterate(self._handle, C.byref(self.bufs), col0, ncol, int(max_iter),
+                                                  float(tolJ), float(tolPops), self._stream()))
 
     def raise_on_faults(self, col0=0, ncol=None):
         """What the reference would have raised during the loop: LinAlgError for a singular statistical-equilibrium
@@ -348,6 +377,22 @@ class MaliEngine:
         self.t_dPops.fill_(1.0)
         self.t_dJ.fill_(1.0)
         self.t_status.zero_()
+        if self.ng is not None:
+            self.t_ng_nse.zero_()
+            self.t_ng_accepted.zero_()
+
+    def ng_reset(self, col0=0, ncol=None):
+        """Restart the Ng history of columns [col0, col0+ncol): needed after their populations were edited between
+        per-call iterations (the extrapolation would otherwise mix the edited vector with the older ones)."""
+        if self.ng is not None:
+            ncol = self.ncol - col0 if ncol is None else ncol
+            self.t_ng_nse[col0:col0 + ncol].zero_()
+
+    def ng_accepted(self):
+        """[ncol, Natom] numpy: Ng extrapolations applied since the last reset_iteration_state (None without Ng)."""
+        if self.ng is None:
+            return None
+        return self.t_ng_accepted.view(self.ncol, self.mt.Natom).cpu().numpy()
 
     # ------------------------------------------------------------------ measurement
     def profile_begin(self, max_launches):
@@ -496,3 +541,18 @@ def fp64_peak(device=None, iters=4096):
     with torch.cuda.device(dev):
         _capi.check(_capi.load().mali_fp64_peak(int(iters), C.c_void_p(scratch.data_ptr()), C.byref(out)))
     return out.value
+
+
+def ng_hook(hist, order, device=None):
+    """One Ng extrapolation with the kernels' own code (test hook of mali_iterate_ng): hist [order+2, nvec], newest
+    first.  Returns (x*, True) if accepted, else (the newest vector, False)."""
+    dev = torch.device('cuda', torch.cuda.current_device() if device is None else device)
+    th = torch.as_tensor(np.ascontiguousarray(hist, dtype=np.float64)).to(dev)
+    if th.dim() != 2 or th.shape[0] != int(order) + 2:
+        raise ValueError('hist must be [order + 2, nvec]')
+    out = torch.empty(th.shape[1], dtype=torch.float64, device=dev)
+    acc = torch.zeros(1, dtype=torch.int32, device=dev)
+    with torch.cuda.device(dev):
+        _capi.check(_capi.load().mali_ng_hook(int(order), th.shape[1], C.c_void_p(th.data_ptr()), C.c_void_p(out.data_ptr()),
+                                              C.c_void_p(acc.data_ptr()), C.c_void_p(torch.cuda.current_stream(dev).cuda_stream)))
+    return out.cpu().numpy(), bool(acc.item())
