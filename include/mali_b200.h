@@ -22,6 +22,7 @@
  *   Background.compute_background_eos background.py:21-53 (witt.py EOS + cop), AtmosphereConstructor.convert_scales
  *   atmosphere.py:70-112 (column mass)                      mali_model_set_eos + mali_background
  *   ComputationalTransition.compute_phi rh_method.py:198-243 mali_compute_phi (device Voigt profiles); mali_line_layout = read-back
+ *   (no reference counterpart; Lightweaver's compute_rays) mali_compute_rays (emergent intensity at user angles)
  *
  * Conventions
  *   - plain C, no exceptions; every function returns 0 on success, a negative MALI_E* code on argument
@@ -67,7 +68,7 @@ typedef struct {
     const double *alpha;       /* concat: continuum cross-sections */
     const double *twohc_l3;    /* concat: 2hc/(NM_TO_M lambda)^3 (continua) */
     const double *wlacont;     /* concat: wlambda/lambda/h (continua) */
-    const double *lambda0;     /* [Ntrans] line-centre wavelength in nm (lines; only read by mali_compute_phi), may be NULL */
+    const double *lambda0;     /* [Ntrans] line-centre wavelength in nm (lines; read by mali_compute_phi / _rays), may be NULL */
 } mali_model_desc;
 
 /* Sizes (in doubles, per column) of every caller-owned array, and the offsets of the reference-layout
@@ -240,6 +241,21 @@ int mali_setup_columns(const mali_model *m, const mali_buffers *bufs, int32_t co
  * calls, is good to ~1e-13, so profiles agree with the reference's to that level, not bit for bit). */
 int mali_compute_phi(const mali_model *m, const mali_buffers *bufs, int32_t col0, int32_t ncol, const double *aDamp,
                      const double *vBroad, const double *vlos, void *stream);
+
+/* Emergent intensity at user angles from the current populations and J, for columns [col0, col0+ncol) (Lightweaver's
+ * Context.compute_rays; the reference has no counterpart).  I_out[c][la][m] is what the NEXT mali_formal_sol_gamma would
+ * return as I[la][mu] if mu[m] were one of the model's quadrature angles: opacity and emissivity from the current n, the
+ * scattering term from the current J (zero after an upload), the line profiles of the up-going direction at mu[m]
+ * (rh_method.py:223-231, the device Voigt function of mali_compute_phi), the thermalised lower boundary.  Always the
+ * exact arithmetic form.  Writes nothing but I_out and bad: the call can sit between any two iterations.
+ *   mu: HOST array [nmu], 0 < mu <= 1, 1 <= nmu <= MALI_RAYS_MAX_MU (carried in the kernel parameters)
+ *   aDamp [ncol][Ntrans][Nspace], vBroad [ncol][Natom][Nspace], vlos [ncol][Nspace]: device, per call (the convention
+ *   of mali_compute_phi; may be NULL for a model without lines).  Needs mali_model_desc.lambda0 when there are lines.
+ *   I_out: device [ncol][Nspect][nmu].  bad: device [ncol] or NULL, bit 1 as in status (the caller zeroes it). */
+#define MALI_RAYS_MAX_MU 64
+int mali_compute_rays(const mali_model *m, const mali_buffers *b, int32_t col0, int32_t ncol, int32_t nmu,
+                      const double *mu, const double *aDamp, const double *vBroad, const double *vlos,
+                      double *I_out, int32_t *bad, void *stream);
 
 /* Context.formal_sol_gamma_matrices for columns [col0, col0+ncol): updates J, I, Gamma and dJ.  J-dagger (the
  * previous call's J; zero after an upload, rh_method.py:541) is kept by the library inside colconst.  Work is

@@ -65,7 +65,9 @@ EXPORTS = ['mali_last_error', 'mali_device_count', 'mali_model_create', 'mali_mo
            'mali_profile_end', 'mali_launch_count', 'mali_fp64_peak', 'mali_line_layout', 'mali_model_set_arith', 'mali_model_get_arith',
            'mali_upload_columns_atmos', 'mali_model_set_atoms', 'mali_setup_columns',
            'mali_upload_columns_thermo', 'mali_model_set_eos', 'mali_background', 'mali_graph_iterations',
-           'mali_ng_layout', 'mali_stat_equil_ng', 'mali_iterate_ng', 'mali_ng_hook']
+           'mali_ng_layout', 'mali_stat_equil_ng', 'mali_iterate_ng', 'mali_ng_hook', 'mali_compute_rays']
+
+RAYS_MAX_MU = 64   # MALI_RAYS_MAX_MU
 
 ARITH_EXACT, ARITH_CONTRACTED = 0, 1
 
@@ -125,6 +127,8 @@ def load(path=None):
     L.mali_iterate_ng.argtypes = [C.c_void_p, C.POINTER(Buffers), C.POINTER(NgBuffers), C.POINTER(NgParams), C.c_int32,
                                   C.c_int32, C.c_int32, C.c_double, C.c_double, C.c_void_p]
     L.mali_ng_hook.argtypes = [C.c_int32, C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
+    L.mali_compute_rays.argtypes = [C.c_void_p, C.POINTER(Buffers), C.c_int32, C.c_int32, C.c_int32, _dp] + \
+        [C.c_void_p] * 6
     L.mali_uv.argtypes = [C.c_void_p, C.POINTER(Buffers)] + [C.c_int32] * 5 + [C.c_void_p] * 4
     _libs[path] = L
     return L

@@ -5,6 +5,7 @@
     dJ = ctx.formal_sol_gamma_matrices()              # rh_method.py:565-708
     dPops = ctx.stat_equil()                          # rh_method.py:710-745
     ctx.I, ctx.J, ctx.activeAtoms[0].n, .Gamma        # same names, shapes and aliasing as the reference
+    I = ctx.compute_rays([1.0, 0.5])                  # [Nspect, nmu]: emergent intensity at user angles (Lightweaver)
 
 Only the hot path moves to the GPU.  Everything in this file is the host-side mirror of the reference's per-Context
 SET-UP (ComputationalTransition / ComputationalAtom construction, rh_method.py:93-131,366-423,474-487): it asks the
@@ -202,6 +203,14 @@ class Context:
         self._pull_pops()
         return dPops
 
+    def compute_rays(self, mus):
+        """Emergent intensity [Nspect, nmu] at the angles `mus` (0 < mu <= 1; a scalar gives nmu = 1) from the current
+        populations (edits through the eqPops alias included) and the current J -- Lightweaver's Context.compute_rays.
+        It is the I the next formal_sol_gamma_matrices() would return if `mus` were the angles of the quadrature
+        (the same line profiles, formed on the GPU at these angles); it changes nothing the iteration uses."""
+        self._push_pops()
+        return self._engine.compute_rays(mus, self._col, 1)[0]
+
     def ng_reset(self):
         """Restart the Ng history (Context(ng=...)): call it after editing populations between iterations."""
         self._engine.ng_reset(self._col, 1)
@@ -272,6 +281,12 @@ class BatchContext:
         for c in self.contexts:
             c._pull_pops()
         return dPops
+
+    def compute_rays(self, mus):
+        """Context.compute_rays for every column: [ncol, Nspect, nmu]."""
+        for c in self.contexts:
+            c._push_pops()
+        return self._engine.compute_rays(mus)
 
     def iterate(self, max_iter=500, tolJ=2e-3, tolPops=1e-3):
         """The loop of test.py:20-29 for every column, kept on the device (mali_iterate): returns the iteration

@@ -15,6 +15,7 @@
 
 #include "../../include/mali_b200.h"
 #include "mali_kernels.cuh"
+#include "mali_rays.cuh"
 #include "mali_fs_launch.h"
 
 using namespace mali;
@@ -189,6 +190,7 @@ struct mali_model {
     PhiTile *d_phiTiles = nullptr;
     PhiLine *d_phiLines = nullptr;
     double *d_wavelength = nullptr, *d_muz = nullptr, *d_wmu = nullptr;
+    double *d_lambda0 = nullptr;        // [Ntrans] line centres (zeros without mali_model_desc.lambda0): mali_compute_rays
     int nPhiLines = 0;
     AtomLevels atoms{};                 // model-level atom data of the device-side set-up (mali_model_set_atoms)
     std::vector<void *> atomDev;
@@ -694,6 +696,9 @@ int mali_model_create(const mali_model_desc *d, int device, mali_model **out)
         up(to_device(wl, &m->d_wavelength));
         up(to_device(mz, &m->d_muz));
         up(to_device(wm, &m->d_wmu));
+        std::vector<double> l0(d->Ntrans, 0.0);
+        if (d->lambda0) l0.assign(d->lambda0, d->lambda0 + d->Ntrans);
+        up(to_device(l0, &m->d_lambda0));
     }
     up(to_device(m->genericTiles, &m->d_genericTiles));
     {
@@ -736,7 +741,7 @@ void mali_model_destroy(mali_model *m)
     void *ptrs[] = {m->d_tiles, m->d_slots, m->d_alpha, m->d_twohc, m->d_wlacont, m->d_wlambda, m->d_zmu, m->d_hw,
                     m->d_Nlevel, m->d_lvlOff, m->d_g2Off, m->d_trans, m->d_trPartOff, m->d_trPartRows,
                     m->d_genericTiles, m->d_cjobs, m->d_pchunks, m->d_ptiles, m->d_pslots, m->d_tileJ, m->d_phiTiles,
-                    m->d_phiLines, m->d_wavelength, m->d_muz, m->d_wmu, m->d_gijCont, m->d_gijTiles, m->d_groupTiles};
+                    m->d_phiLines, m->d_wavelength, m->d_muz, m->d_wmu, m->d_gijCont, m->d_gijTiles, m->d_groupTiles, m->d_lambda0};
     for (void *p : ptrs)
         if (p) cudaFree(p);
     for (void *p : m->atomDev)
@@ -1027,6 +1032,64 @@ int mali_compute_phi(const mali_model *m, const mali_buffers *b, int32_t col0, i
         m->d_phiLines, m->d_phiTiles, m->d_wavelength, m->d_wlambda, m->d_muz, m->d_wmu,
         m->N, m->Nrays, m->Nspect, m->Lw, m->Ntrans, m->Natom, aDamp, vBroad, vlos, b->colconst, m->lay.colconst, m->off_tab,
         col0);
+    m->launches += 1;
+    CU(cudaGetLastError());
+    return MALI_OK;
+}
+
+int mali_compute_rays(const mali_model *m, const mali_buffers *b, int32_t col0, int32_t ncol, int32_t nmu, const double *mu,
+                      const double *aDamp, const double *vBroad, const double *vlos, double *I_out, int32_t *bad, void *stream)
+{
+    if (int r = check_range(m, b, col0, ncol, "mali_compute_rays")) return r;
+    if (!b->colconst || !b->pops || !b->J || !I_out) return fail(MALI_EINVAL, "mali_compute_rays: null buffer");
+    if (nmu < 1 || nmu > MALI_RAYS_MAX_MU || !mu)
+        return fail(MALI_EINVAL, "mali_compute_rays: nmu=%d not in [1, %d] (or no angles)", nmu, MALI_RAYS_MAX_MU);
+    for (int q = 0; q < nmu; ++q)
+        if (!(mu[q] > 0.0 && mu[q] <= 1.0)) return fail(MALI_EINVAL, "mali_compute_rays: mu[%d]=%g not in (0, 1]", q, mu[q]);
+    if (m->nPhiLines > 0) {   // the line profiles are formed at the new angles from the per-call inputs
+        if (!m->haveLambda0) return fail(MALI_EINVAL, "mali_compute_rays: the model was created without lambda0");
+        if (!aDamp || !vBroad || !vlos) return fail(MALI_EINVAL, "mali_compute_rays: null aDamp / vBroad / vlos");
+    }
+    static_assert(kRaysMaxMu == MALI_RAYS_MAX_MU, "mali_rays.cuh and mali_b200.h disagree on the angle limit");
+    RaysParams p{};
+    p.N = m->N;
+    p.Nrays = m->Nrays;
+    p.Nspect = m->Nspect;
+    p.Natom = m->Natom;
+    p.Ntrans = m->Ntrans;
+    p.Lw = m->Lw;
+    p.ntile = m->ntile;
+    p.nchunk = (nmu + m->Nrays - 1) / m->Nrays;
+    p.nmu = nmu;
+    p.col0 = col0;
+    p.ncol = ncol;
+    p.colStride = m->lay.colconst;
+    p.popStride = m->lay.pops;
+    p.JStride = m->lay.J;
+    p.off_z = m->off_z;
+    p.off_bbc = m->off_bbc;
+    p.off_tab = m->off_tab;
+    p.tiles = m->d_tiles;
+    p.slots = m->d_slots;
+    p.alpha = m->d_alpha;
+    p.twohc = m->d_twohc;
+    p.wavelength = m->d_wavelength;
+    p.lambda0 = m->d_lambda0;
+    p.colconst = b->colconst;
+    p.pops = b->pops;
+    p.J = b->J;
+    p.aDamp = aDamp;
+    p.vBroad = vBroad;
+    p.vlos = vlos;
+    p.I = I_out;
+    p.bad = bad;
+    for (int q = 0; q < nmu; ++q) {
+        p.mu[q] = mu[q];
+        p.zmu[q] = 1.0 / mu[q];   // formal_solver.py:92, as mali_model_create forms zmu
+    }
+    const int64_t warps = (int64_t)ncol * m->ntile * p.nchunk;
+    const int wpb = 4;
+    rays_kernel<<<(unsigned)((warps + wpb - 1) / wpb), 32 * wpb, 0, (cudaStream_t)stream>>>(p);
     m->launches += 1;
     CU(cudaGetLastError());
     return MALI_OK;

@@ -6,6 +6,7 @@ radiative model, and drives libmali_b200.so through its C ABI.
     dJ = eng.formal_sol_gamma_matrices()                  # [ncol] numpy   (rh_method.py:565-708)
     dP = eng.stat_equil()                                 # [ncol] numpy   (rh_method.py:710-745)
     eng.J(col), eng.I(col), eng.Gamma(col), eng.n(col)    # numpy, reference shapes
+    I = eng.compute_rays([1.0, 0.5])                      # [ncol, Nspect, nmu] emergent intensity at user angles
 
 Columns are independent (no cross-column arithmetic anywhere), which is what makes the path data-parallel:
 ranks of a multi-GPU job each own a contiguous slice of columns (see lightspinner_b200/sharding.py).
@@ -72,6 +73,14 @@ class MaliEngine:
         self.bufs = _capi.Buffers(n, *(t.data_ptr() for t in (
             self.t_colconst, self.t_pops, self.t_J, self.t_I, self.t_Gamma, self.t_scratch, self.t_dJ,
             self.t_dPops, self.t_status, self.t_iter, self.t_done)))
+        # each column's line-profile inputs, kept for compute_rays (which forms the profiles at new angles); the
+        # uploads that take host profiles instead leave a column without them (_has_profile False)
+        N = self.mt.Nspace
+        self.t_aDamp = torch.zeros(n, self.mt.Ntrans, N, **f64)
+        self.t_vBroad = torch.zeros(n, self.mt.Natom, N, **f64)
+        self.t_vlos = torch.zeros(n, N, **f64)
+        self._has_profile = np.zeros(n, dtype=bool)
+        self._rays_bad = None
         self.chunk = max(1, min(int(max_upload_chunk), n))
         self._staging = None
         self._pinned = None
@@ -142,7 +151,30 @@ class MaliEngine:
             for q, p in enumerate(chunk):
                 pack_column(self.mt, self.lay, p, out=pin_np[q * hp:(q + 1) * hp])
             self.upload_packed(pinned, col0 + c0, len(chunk))
+            for q, p in enumerate(chunk):    # keep the profile inputs when the dict carries them
+                if all(k in p for k in ('aDamp', 'vBroad', 'vlos')):
+                    self._keep_profile_inputs(col0 + c0 + q, 1, *(np.asarray(p[k], dtype=np.float64)[None]
+                                                                  for k in ('aDamp', 'vBroad', 'vlos')))
         torch.cuda.current_stream(self.device).synchronize()
+
+    def _keep_profile_inputs(self, col0, ncol, aDamp, vBroad, vlos):
+        """Copies a range of columns' aDamp / vBroad / vlos (numpy arrays or device tensors) into the persistent
+        tensors compute_rays reads, and returns those slices.  Inputs that are not of the model's shape (e.g. the aDamp
+        rows of lines a derived model dropped; compute_phi reads nothing of a model without lines) are not kept: the
+        columns are then marked as having no profile inputs and None is returned."""
+        c1 = col0 + ncol
+        ins = [torch.as_tensor(a, dtype=torch.float64) for a in (aDamp, vBroad, vlos)]
+        if any(a.numel() != ncol * t[0].numel() for a, t in zip(ins, (self.t_aDamp, self.t_vBroad, self.t_vlos))):
+            self._has_profile[col0:c1] = False
+            return None
+        out = []
+        for t, a in zip((self.t_aDamp, self.t_vBroad, self.t_vlos), ins):
+            dst = t[col0:c1]
+            if a.data_ptr() != dst.data_ptr() or a.device != dst.device:
+                dst.copy_(a.reshape(dst.shape), non_blocking=a.device == dst.device)
+            out.append(dst)
+        self._has_profile[col0:c1] = True
+        return out
 
     def upload_device_phi(self, problems, col0=0):
         """Like upload(), but the Voigt line profiles are formed on the device (ComputationalTransition.compute_phi,
@@ -163,7 +195,7 @@ class MaliEngine:
                    for k in ('aDamp', 'vBroad', 'vlos')]
             if aux[0].shape[1] != self.mt.Ntrans or aux[1].shape[1] != self.mt.Natom or aux[2].shape[1] != 1:
                 raise ValueError('aDamp / vBroad / vlos must be [Ntrans, Nspace] / [Natom, Nspace] / [Nspace]')
-            dev = [torch.from_numpy(np.ascontiguousarray(a)).to(self.device) for a in aux]
+            dev = self._keep_profile_inputs(col0 + c0, len(chunk), *aux)      # (shapes checked above)
             with torch.cuda.device(self.device):
                 self._check(self.lib.mali_upload_columns_nophi(self._handle, C.byref(self.bufs), col0 + c0, len(chunk),
                                                                C.c_void_p(pinned.data_ptr()),
@@ -201,7 +233,9 @@ class MaliEngine:
             aux = {k: torch.from_numpy(np.ascontiguousarray(np.stack(
                 [np.asarray(p[k], dtype=np.float64).reshape(-1, N) for p in chunk]))).to(self.device)
                 for k in ('temperature', 'ne', 'vturb', 'vlos', 'aDamp')}
-            vBroad = torch.empty((nc, self.mt.Natom, N), dtype=torch.float64, device=self.device)
+            # mali_setup_columns writes the Doppler widths straight into the persistent slice compute_rays reads
+            vBroad = self.t_vBroad[col0 + c0:col0 + c0 + nc]
+            self._keep_profile_inputs(col0 + c0, nc, aux['aDamp'], vBroad, aux['vlos'])
             ns = self.nStar[(col0 + c0) * self.lay.sumNlevel * N:(col0 + c0 + nc) * self.lay.sumNlevel * N]
             P = lambda t: C.c_void_p(t.data_ptr())
             with torch.cuda.device(self.device):
@@ -247,7 +281,8 @@ class MaliEngine:
             keys = ['temperature', 'ne', 'nHTot', 'vturb', 'vlos', 'aDamp'] + (['cmass'] if 'cmass' in chunk[0] else [])
             aux = {k: torch.from_numpy(np.ascontiguousarray(np.stack(
                 [np.asarray(p[k], dtype=np.float64).reshape(-1, N) for p in chunk]))).to(self.device) for k in keys}
-            vBroad = torch.empty((nc, self.mt.Natom, N), dtype=torch.float64, device=self.device)
+            vBroad = self.t_vBroad[col0 + c0:col0 + c0 + nc]
+            self._keep_profile_inputs(col0 + c0, nc, aux['aDamp'], vBroad, aux['vlos'])
             work = torch.empty(nc * N * 21, dtype=torch.float64, device=self.device)
             ns = self.nStar[(col0 + c0) * self.lay.sumNlevel * N:(col0 + c0 + nc) * self.lay.sumNlevel * N]
             P = lambda t: C.c_void_p(t.data_ptr())
@@ -273,6 +308,7 @@ class MaliEngine:
         """Asynchronous form of upload_device_phi: `host_prefix_pinned` holds [ncol][lay.hp_phi] doubles (pinned),
         aDamp / vBroad / vlos are device tensors [ncol][Ntrans|Natom|1][Nspace]."""
         self.ng_reset(col0, ncol)
+        self._keep_profile_inputs(col0, ncol, aDamp, vBroad, vlos)
         if staging is None:
             staging, _ = self._staging_bufs(0)
         if ncol * self.lay.hostpack > staging.numel():
@@ -286,8 +322,11 @@ class MaliEngine:
                                                   C.c_void_p(vlos.data_ptr()), self._stream()))
 
     def upload_packed(self, host_pinned, col0, ncol, staging=None):
-        """H2D copy of `ncol` host-pack blocks (a pinned torch tensor) + device re-layout; asynchronous."""
+        """H2D copy of `ncol` host-pack blocks (a pinned torch tensor) + device re-layout; asynchronous.  The blocks
+        carry the line profiles, not their inputs: compute_rays refuses these columns (upload() keeps the inputs
+        when the problem dicts have them)."""
         self.ng_reset(col0, ncol)
+        self._has_profile[col0:col0 + ncol] = False
         if staging is None:
             staging, _ = self._staging_bufs(0)
         if ncol * self.lay.hostpack > staging.numel():
@@ -300,6 +339,7 @@ class MaliEngine:
     def repack_from_staging(self, staging, col0, ncol):
         """Device re-layout only (the staging tensor already holds host-pack blocks on the device)."""
         self.ng_reset(col0, ncol)
+        self._has_profile[col0:col0 + ncol] = False
         with torch.cuda.device(self.device):
             self._check(self.lib.mali_upload_columns(self._handle, C.byref(self.bufs), col0, ncol, None,
                                                      C.c_void_p(staging.data_ptr()), self._stream()))
@@ -370,6 +410,55 @@ class MaliEngine:
             bad = col0 + np.nonzero((status & 2) | (done == 2))[0]
             raise FloatingPointError('non-finite result or opacity / optical-depth step outside the formal solver\'s '
                                      'numeric domain in column(s) %s' % bad[:8].tolist())
+
+    # ------------------------------------------------------------------ emergent intensity at user angles
+    def compute_rays_async(self, mus, col0=0, ncol=None, out=None):
+        """Emergent intensity at the angles `mus` (0 < mu <= 1; a scalar is one angle) from the current populations and
+        J of columns [col0, col0+ncol) (mali_compute_rays): a device tensor [ncol, Nspect, nmu], `out` if given.  It is
+        what the next formal solution would return as I if those angles were its quadrature angles; nothing else is
+        written, so it can be called between any two iterations.  Lists longer than MALI_RAYS_MAX_MU are split into
+        several launches.  Domain faults are collected for compute_rays (see there)."""
+        mus = rays_angles(mus)
+        ncol = self.ncol - col0 if ncol is None else ncol
+        if col0 < 0 or ncol < 1 or col0 + ncol > self.ncol:
+            raise ValueError('columns [%d, %d) outside the batch of %d' % (col0, col0 + ncol, self.ncol))
+        if (self.mt.trans[:, 3] != 0).any() and not self._has_profile[col0:col0 + ncol].all():
+            bad = col0 + np.nonzero(~self._has_profile[col0:col0 + ncol])[0]
+            raise ValueError('column(s) %s were uploaded with host line profiles and without their inputs (aDamp, vBroad, '
+                             'vlos): compute_rays needs those to form the profiles at new angles' % bad[:8].tolist())
+        nmu, S = mus.shape[0], self.mt.Nspect
+        if out is None:
+            out = torch.empty(ncol, S, nmu, dtype=torch.float64, device=self.device)
+        elif (tuple(out.shape) != (ncol, S, nmu) or out.dtype != torch.float64 or out.device != self.device
+              or not out.is_contiguous()):
+            raise ValueError('out must be a contiguous float64 tensor [%d, %d, %d] on %s' % (ncol, S, nmu, self.device))
+        self._rays_bad = torch.zeros(ncol, dtype=torch.int32, device=self.device)
+        P = lambda t: C.c_void_p(t.data_ptr()) if t.numel() else None
+        args = [P(self.t_aDamp[col0:]), P(self.t_vBroad[col0:]), P(self.t_vlos[col0:])]
+        step = _capi.RAYS_MAX_MU
+        with torch.cuda.device(self.device):
+            for q0 in range(0, nmu, step):
+                part = mus[q0:q0 + step]
+                dst = out if nmu <= step else torch.empty(ncol, S, part.shape[0], dtype=torch.float64, device=self.device)
+                self._check(self.lib.mali_compute_rays(self._handle, C.byref(self.bufs), col0, ncol, part.shape[0],
+                                                       part.ctypes.data_as(C.POINTER(C.c_double)), *args, P(dst),
+                                                       P(self._rays_bad), self._stream()))
+                if dst is not out:
+                    out[:, :, q0:q0 + part.shape[0]].copy_(dst)
+        return out
+
+    def compute_rays(self, mus, col0=0, ncol=None):
+        """compute_rays_async as numpy [ncol, Nspect, nmu]; raises FloatingPointError if an opacity / optical-depth step
+        of a column left the formal solver's numeric domain (status bit 1 of the formal solution)."""
+        col0 = int(col0)
+        out = self.compute_rays_async(mus, col0, ncol)
+        res = out.cpu().numpy()
+        bad = self._rays_bad.cpu().numpy()
+        if (bad & 2).any():
+            cols = col0 + np.nonzero(bad & 2)[0]
+            raise FloatingPointError('opacity or optical-depth step outside the formal solver\'s numeric domain '
+                                     '(zero, subnormal, infinite or NaN) in column(s) %s' % cols[:8].tolist())
+        return res
 
     def reset_iteration_state(self):
         self.t_iter.zero_()
@@ -487,6 +576,20 @@ class MaliEngine:
                                          C.c_void_p(out[2].data_ptr()), self._stream()))
         o = out.cpu().numpy()
         return o[0], o[1], o[2]   # Uji, Vij, Vji
+
+
+def rays_angles(mus):
+    """The angles of a compute_rays call as a 1-D float64 array: a scalar is one angle; every angle must be finite
+    and in (0, 1] (ValueError otherwise)."""
+    a = np.asarray(mus, dtype=np.float64)
+    if a.ndim == 0:
+        a = a.reshape(1)
+    if a.ndim != 1 or a.shape[0] == 0:
+        raise ValueError('mus must be a scalar or a non-empty 1-D sequence of angles, got shape %s' % (a.shape,))
+    ok = np.isfinite(a) & (a > 0.0) & (a <= 1.0)
+    if not ok.all():
+        raise ValueError('every mu must lie in (0, 1]: got %s' % a[~ok][:8].tolist())
+    return np.ascontiguousarray(a)
 
 
 def piecewise_linear_1d_batch(z, muz, toFrom, bbc0, bbc1, chi, S, device=None):
