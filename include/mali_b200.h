@@ -23,6 +23,8 @@
  *   atmosphere.py:70-112 (column mass)                      mali_model_set_eos + mali_background
  *   ComputationalTransition.compute_phi rh_method.py:198-243 mali_compute_phi (device Voigt profiles); mali_line_layout = read-back
  *   (no reference counterpart; Lightweaver's compute_rays) mali_compute_rays (emergent intensity at user angles)
+ *   (no reference counterpart; Lightweaver's depthData)    mali_compute_rays_depth (I, chi, S, tau, contribution
+ *                                                           function, tau = 1 heights along those rays)
  *
  * Conventions
  *   - plain C, no exceptions; every function returns 0 on success, a negative MALI_E* code on argument
@@ -256,6 +258,36 @@ int mali_compute_phi(const mali_model *m, const mali_buffers *bufs, int32_t col0
 int mali_compute_rays(const mali_model *m, const mali_buffers *b, int32_t col0, int32_t ncol, int32_t nmu,
                       const double *mu, const double *aDamp, const double *vBroad, const double *vlos,
                       double *I_out, int32_t *bad, void *stream);
+
+/* Depth-resolved data of the up-going rays mali_compute_rays sweeps (Lightweaver's ctx.depthData): same state, inputs,
+ * angles, argument checks and exact arithmetic; writes nothing but the requested outputs and bad.  Device pointers,
+ * each may be NULL (at least one must be given).  Depth arrays are [ncol][Nspace][Nspect][nmu], depth k = 0 at the top:
+ *   chi[k]      the total opacity the sweep uses at k (line and continuum slots, then the background)
+ *   S[k]        the source function the sweep uses at k
+ *   I[k]        the up-going intensity at k: I[Nspace-1] is the thermalised boundary value, I[0] is bit-identical to
+ *               mali_compute_rays' output
+ *   tau[k]      optical depth along the ray from the top: tau[0] = 0, tau[k] = tau[k-1] + dtau[k-1], summed top down,
+ *               dtau[j] the step between depths j and j+1 exactly as the sweep forms it (bit-identical to the oracle's
+ *               0.5*(chi[j]+chi[j+1])*zmu*fabs(z[j]-z[j+1]))
+ *   contrib[k]  the contribution of depth k to the emergent intensity, through what each short-characteristic step
+ *               applied: for the step into k (k = Nspace-2 .. 1), (w0, w1) = w2(dtau[k]), delta[k] = w0*S[k] + w1*dS
+ *               (in that order; dS = (S[k+1]-S[k])/dtau[k], the sweep's upwind slope) and a[k] = 1 - w0.  At k = 0 the
+ *               reference's stale-w quirk (formal_solver.py:137-139): w0, w1 and a of the step into 1, with S[1] in
+ *               place of S[0] and dS = (S[1]-S[0])/dtau[0].  delta[Nspace-1] = I[Nspace-1].  T[0] = 1,
+ *               T[k] = T[k-1]*a[k-1] (top down); contrib[k] = delta[k]*T[k].  Sum_k contrib[k] = I[0] in exact
+ *               arithmetic (the recurrence telescopes).
+ * and, per ray, z_tau1 [ncol][Nspect][nmu]: the height of tau = 1.  With k* the first k where tau[k] >= 1,
+ *   z_tau1 = z[k*-1] + (z[k*]-z[k*-1]) * ((1.0 - tau[k*-1]) / (tau[k*]-tau[k*-1])) (IEEE division); NaN if the ray never
+ *   reaches tau = 1.
+ * height [ncol][Nspace]: the column's heights as the formal solution reads them (device-formed for columns set up
+ *   by mali_upload_columns_thermo).
+ * contrib and z_tau1 need tau (MALI_EINVAL otherwise). */
+typedef struct {
+    double *I, *chi, *S, *tau, *contrib, *z_tau1, *height;
+} mali_rays_depth_out;
+int mali_compute_rays_depth(const mali_model *m, const mali_buffers *b, int32_t col0, int32_t ncol, int32_t nmu,
+                            const double *mu, const double *aDamp, const double *vBroad, const double *vlos,
+                            const mali_rays_depth_out *out, int32_t *bad, void *stream);
 
 /* Context.formal_sol_gamma_matrices for columns [col0, col0+ncol): updates J, I, Gamma and dJ.  J-dagger (the
  * previous call's J; zero after an upload, rh_method.py:541) is kept by the library inside colconst.  Work is

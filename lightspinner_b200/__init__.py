@@ -3,21 +3,22 @@
     from lightspinner_b200 import Context, piecewise_linear_1d      # drop-ins for rh_method.Context / formal_solver
     from lightspinner_b200 import MaliEngine                        # batched columns on one GPU
     from lightspinner_b200 import NgOptions                         # opt-in Ng acceleration (ng=NgOptions())
+    from lightspinner_b200 import RayDepthData                      # what compute_rays_depth returns
 
 The compute lives in csrc/ (hand-written CUDA for sm_100a behind the C ABI of include/mali_b200.h); there is no CPU
 fallback.  Importing the package does not touch the GPU; constructing a Context / MaliEngine does.
 """
 
-__all__ = ['Context', 'BatchContext', 'piecewise_linear_1d', 'IPsi', 'UV', 'MaliEngine', 'NgOptions']
+__all__ = ['Context', 'BatchContext', 'piecewise_linear_1d', 'IPsi', 'UV', 'MaliEngine', 'NgOptions', 'RayDepthData']
 
 
 def __getattr__(name):
     if name in ('Context', 'BatchContext', 'piecewise_linear_1d', 'IPsi', 'UV'):
         from . import context
         return getattr(context, name)
-    if name == 'MaliEngine':
-        from .engine import MaliEngine
-        return MaliEngine
+    if name in ('MaliEngine', 'RayDepthData'):
+        from . import engine
+        return getattr(engine, name)
     if name == 'NgOptions':
         from .ng import NgOptions
         return NgOptions

@@ -51,6 +51,10 @@ class Buffers(C.Structure):
                 ('dPops', C.c_void_p), ('status', C.c_void_p), ('iter', C.c_void_p), ('done', C.c_void_p)]
 
 
+class RaysDepthOut(C.Structure):
+    _fields_ = [(n, C.c_void_p) for n in ('I', 'chi', 'S', 'tau', 'contrib', 'z_tau1', 'height')]
+
+
 class NgParams(C.Structure):
     _fields_ = [('order', C.c_int32), ('delay', C.c_int32), ('period', C.c_int32)]
 
@@ -65,7 +69,8 @@ EXPORTS = ['mali_last_error', 'mali_device_count', 'mali_model_create', 'mali_mo
            'mali_profile_end', 'mali_launch_count', 'mali_fp64_peak', 'mali_line_layout', 'mali_model_set_arith', 'mali_model_get_arith',
            'mali_upload_columns_atmos', 'mali_model_set_atoms', 'mali_setup_columns',
            'mali_upload_columns_thermo', 'mali_model_set_eos', 'mali_background', 'mali_graph_iterations',
-           'mali_ng_layout', 'mali_stat_equil_ng', 'mali_iterate_ng', 'mali_ng_hook', 'mali_compute_rays']
+           'mali_ng_layout', 'mali_stat_equil_ng', 'mali_iterate_ng', 'mali_ng_hook', 'mali_compute_rays',
+           'mali_compute_rays_depth']
 
 RAYS_MAX_MU = 64   # MALI_RAYS_MAX_MU
 
@@ -129,6 +134,8 @@ def load(path=None):
     L.mali_ng_hook.argtypes = [C.c_int32, C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
     L.mali_compute_rays.argtypes = [C.c_void_p, C.POINTER(Buffers), C.c_int32, C.c_int32, C.c_int32, _dp] + \
         [C.c_void_p] * 6
+    L.mali_compute_rays_depth.argtypes = [C.c_void_p, C.POINTER(Buffers), C.c_int32, C.c_int32, C.c_int32, _dp] + \
+        [C.c_void_p] * 3 + [C.POINTER(RaysDepthOut), C.c_void_p, C.c_void_p]
     L.mali_uv.argtypes = [C.c_void_p, C.POINTER(Buffers)] + [C.c_int32] * 5 + [C.c_void_p] * 4
     _libs[path] = L
     return L

@@ -6,6 +6,7 @@
     dPops = ctx.stat_equil()                          # rh_method.py:710-745
     ctx.I, ctx.J, ctx.activeAtoms[0].n, .Gamma        # same names, shapes and aliasing as the reference
     I = ctx.compute_rays([1.0, 0.5])                  # [Nspect, nmu]: emergent intensity at user angles (Lightweaver)
+    d = ctx.compute_rays_depth([1.0, 0.5])            # RayDepthData: I, chi, S, tau, contrib [Nspace, Nspect, nmu], ...
 
 Only the hot path moves to the GPU.  Everything in this file is the host-side mirror of the reference's per-Context
 SET-UP (ComputationalTransition / ComputationalAtom construction, rh_method.py:93-131,366-423,474-487): it asks the
@@ -211,6 +212,13 @@ class Context:
         self._push_pops()
         return self._engine.compute_rays(mus, self._col, 1)[0]
 
+    def compute_rays_depth(self, mus, quantities=None):
+        """Depth-resolved data of the rays compute_rays(mus) sweeps (Lightweaver's ctx.depthData), from the same state:
+        a RayDepthData with I, chi, S, tau, contrib [Nspace, Nspect, nmu] (depth 0 at the top), z_tau1 [Nspect, nmu]
+        and the heights [Nspace] (see MaliEngine.compute_rays_depth; `quantities` selects a subset)."""
+        self._push_pops()
+        return self._engine.compute_rays_depth(mus, self._col, 1, quantities).column(0)
+
     def ng_reset(self):
         """Restart the Ng history (Context(ng=...)): call it after editing populations between iterations."""
         self._engine.ng_reset(self._col, 1)
@@ -287,6 +295,12 @@ class BatchContext:
         for c in self.contexts:
             c._push_pops()
         return self._engine.compute_rays(mus)
+
+    def compute_rays_depth(self, mus, quantities=None):
+        """Context.compute_rays_depth for every column: a RayDepthData with a leading column axis."""
+        for c in self.contexts:
+            c._push_pops()
+        return self._engine.compute_rays_depth(mus, quantities=quantities)
 
     def iterate(self, max_iter=500, tolJ=2e-3, tolPops=1e-3):
         """The loop of test.py:20-29 for every column, kept on the device (mali_iterate): returns the iteration

@@ -1037,21 +1037,24 @@ int mali_compute_phi(const mali_model *m, const mali_buffers *b, int32_t col0, i
     return MALI_OK;
 }
 
-int mali_compute_rays(const mali_model *m, const mali_buffers *b, int32_t col0, int32_t ncol, int32_t nmu, const double *mu,
-                      const double *aDamp, const double *vBroad, const double *vlos, double *I_out, int32_t *bad, void *stream)
+// The argument checks of mali_compute_rays and mali_compute_rays_depth, and the kernel parameters they share (the
+// outputs are left null for the caller to set).
+static int rays_params(const mali_model *m, const mali_buffers *b, int32_t col0, int32_t ncol, int32_t nmu,
+                       const double *mu, const double *aDamp, const double *vBroad, const double *vlos, int32_t *bad,
+                       const char *who, RaysParams &p)
 {
-    if (int r = check_range(m, b, col0, ncol, "mali_compute_rays")) return r;
-    if (!b->colconst || !b->pops || !b->J || !I_out) return fail(MALI_EINVAL, "mali_compute_rays: null buffer");
+    if (int r = check_range(m, b, col0, ncol, who)) return r;
+    if (!b->colconst || !b->pops || !b->J) return fail(MALI_EINVAL, "%s: null buffer", who);
     if (nmu < 1 || nmu > MALI_RAYS_MAX_MU || !mu)
-        return fail(MALI_EINVAL, "mali_compute_rays: nmu=%d not in [1, %d] (or no angles)", nmu, MALI_RAYS_MAX_MU);
+        return fail(MALI_EINVAL, "%s: nmu=%d not in [1, %d] (or no angles)", who, nmu, MALI_RAYS_MAX_MU);
     for (int q = 0; q < nmu; ++q)
-        if (!(mu[q] > 0.0 && mu[q] <= 1.0)) return fail(MALI_EINVAL, "mali_compute_rays: mu[%d]=%g not in (0, 1]", q, mu[q]);
+        if (!(mu[q] > 0.0 && mu[q] <= 1.0)) return fail(MALI_EINVAL, "%s: mu[%d]=%g not in (0, 1]", who, q, mu[q]);
     if (m->nPhiLines > 0) {   // the line profiles are formed at the new angles from the per-call inputs
-        if (!m->haveLambda0) return fail(MALI_EINVAL, "mali_compute_rays: the model was created without lambda0");
-        if (!aDamp || !vBroad || !vlos) return fail(MALI_EINVAL, "mali_compute_rays: null aDamp / vBroad / vlos");
+        if (!m->haveLambda0) return fail(MALI_EINVAL, "%s: the model was created without lambda0", who);
+        if (!aDamp || !vBroad || !vlos) return fail(MALI_EINVAL, "%s: null aDamp / vBroad / vlos", who);
     }
     static_assert(kRaysMaxMu == MALI_RAYS_MAX_MU, "mali_rays.cuh and mali_b200.h disagree on the angle limit");
-    RaysParams p{};
+    p = RaysParams{};
     p.N = m->N;
     p.Nrays = m->Nrays;
     p.Nspect = m->Nspect;
@@ -1081,18 +1084,58 @@ int mali_compute_rays(const mali_model *m, const mali_buffers *b, int32_t col0, 
     p.aDamp = aDamp;
     p.vBroad = vBroad;
     p.vlos = vlos;
-    p.I = I_out;
     p.bad = bad;
     for (int q = 0; q < nmu; ++q) {
         p.mu[q] = mu[q];
         p.zmu[q] = 1.0 / mu[q];   // formal_solver.py:92, as mali_model_create forms zmu
     }
-    const int64_t warps = (int64_t)ncol * m->ntile * p.nchunk;
+    return MALI_OK;
+}
+
+static int launch_rays(const mali_model *m, const RaysParams &p, bool depth, void *stream)
+{
+    const int64_t warps = (int64_t)p.ncol * p.ntile * p.nchunk;
     const int wpb = 4;
-    rays_kernel<<<(unsigned)((warps + wpb - 1) / wpb), 32 * wpb, 0, (cudaStream_t)stream>>>(p);
+    (depth ? rays_kernel<true> : rays_kernel<false>)<<<(unsigned)((warps + wpb - 1) / wpb), 32 * wpb, 0, (cudaStream_t)stream>>>(p);
     m->launches += 1;
     CU(cudaGetLastError());
     return MALI_OK;
+}
+
+int mali_compute_rays(const mali_model *m, const mali_buffers *b, int32_t col0, int32_t ncol, int32_t nmu, const double *mu,
+                      const double *aDamp, const double *vBroad, const double *vlos, double *I_out, int32_t *bad, void *stream)
+{
+    RaysParams p;
+    if (int r = rays_params(m, b, col0, ncol, nmu, mu, aDamp, vBroad, vlos, bad, "mali_compute_rays", p)) return r;
+    if (!I_out) return fail(MALI_EINVAL, "mali_compute_rays: null buffer");
+    p.I = I_out;
+    return launch_rays(m, p, false, stream);
+}
+
+int mali_compute_rays_depth(const mali_model *m, const mali_buffers *b, int32_t col0, int32_t ncol, int32_t nmu,
+                            const double *mu, const double *aDamp, const double *vBroad, const double *vlos,
+                            const mali_rays_depth_out *out, int32_t *bad, void *stream)
+{
+    RaysParams p;
+    if (int r = rays_params(m, b, col0, ncol, nmu, mu, aDamp, vBroad, vlos, bad, "mali_compute_rays_depth", p)) return r;
+    if (!out || !(out->I || out->chi || out->S || out->tau || out->contrib || out->z_tau1 || out->height))
+        return fail(MALI_EINVAL, "mali_compute_rays_depth: no output requested");
+    if ((out->contrib || out->z_tau1) && !out->tau)
+        return fail(MALI_EINVAL, "mali_compute_rays_depth: contrib and z_tau1 need the tau buffer");
+    if (out->height) {   // the heights the sweep reads: colconst's z rows
+        const size_t N = (size_t)m->N;
+        CU(cudaMemcpy2DAsync(out->height, N * sizeof(double), b->colconst + (size_t)col0 * m->lay.colconst + m->off_z,
+                             (size_t)m->lay.colconst * sizeof(double), N * sizeof(double), (size_t)ncol,
+                             cudaMemcpyDeviceToDevice, (cudaStream_t)stream));
+    }
+    if (!(out->I || out->chi || out->S || out->tau)) return MALI_OK;
+    p.dI = out->I;
+    p.dchi = out->chi;
+    p.dS = out->S;
+    p.dtau = out->tau;
+    p.dcontrib = out->contrib;
+    p.ztau1 = out->z_tau1;
+    return launch_rays(m, p, true, stream);
 }
 
 static FsParams make_fs_params(const mali_model *m, const mali_buffers *b, int col0, int ncol, int wpb)

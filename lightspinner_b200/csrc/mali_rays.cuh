@@ -7,6 +7,11 @@
 // compute_phi_kernel's expressions (rh_method.py:223-231), and the up sweep of the generic kernel (thermalised lower
 // boundary, the last-point quirk of formal_solver.py:137-139).  Always the exact arithmetic form (Arith<false>).
 // Nothing but I_out and the optional fault word is written.
+//
+// rays_kernel<true> (mali_compute_rays_depth) runs the same up sweep and also stores, per depth, what the sweep used:
+// chi, S and I, the optical-depth step into each depth (in the tau buffer) and each step's source term delta (in the
+// contrib buffer).  A second pass of the same lane, top down, turns the steps into tau and delta into the contribution
+// function, and finds the height of tau = 1 (definitions in include/mali_b200.h).
 #pragma once
 #include "mali_device.cuh"
 
@@ -26,11 +31,15 @@ struct RaysParams {
     double *I;                             // [ncol][Nspect][nmu]
     int32_t *bad;                          // [ncol] or null: bit 1 as in mali_buffers.status
     double mu[kRaysMaxMu], zmu[kRaysMaxMu];   // the angles and 1/mu (host: 1.0 / mu, as mali_model_create forms zmu)
+    // rays_kernel<true> only, each may be null (appended, so every field rays_kernel<false> reads keeps its offset).
+    // dI, dchi, dS, dtau, dcontrib: [ncol][N][Nspect][nmu]; ztau1: [ncol][Nspect][nmu].  dcontrib and ztau1 need dtau.
+    double *dI, *dchi, *dS, *dtau, *dcontrib, *ztau1;
 };
 
 // One warp per (column, wavelength tile, mu-chunk), the lane mapping of the formal-solution kernels: ls = lane / Nrays,
 // angle = chunk * Nrays + lane % Nrays.  Per lane the up sweep of one ray, in registers: no Gamma, no J, no shared memory
 // and no warp-collective operation, so lanes without a ray leave at once.
+template <bool DEPTH>
 __global__ void __launch_bounds__(128) rays_kernel(const RaysParams p)
 {
     const int lane = threadIdx.x & 31;
@@ -111,15 +120,73 @@ __global__ void __launch_bounds__(128) rays_kernel(const RaysParams p)
         const double rchi = rcp_full(chiTot);
         const double S = div_by(etaTot + __ldg(bg + Lw) + __ldg(bg + 2 * Lw) * Jdag, chiTot, rchi);
 
+        // ---- the step into k as step() forms it: dtau[k] (between k+1 and k), the upwind slope, and S' (S[k]; S[1] at
+        // k = 0, formal_solver.py:137-139).  Read before step() moves chiPrev / SPrev / zPrev on.
+        double dtau = 0.0, dS = 0.0, Sw = S;
+        if constexpr (DEPTH) {
+            if (s > 0) {
+                dtau = ((sw.chiPrev + chiTot) * (0.5 * zmu)) * fabs(sw.zPrev - zz[k]);
+                dS = div_by(sw.SPrev - S, dtau, rcp_full(dtau));
+                if (s == N - 1) Sw = sw.SPrev;
+            }
+        }
+
         // ---- short characteristic, up-going: formal_solver.py
         double Ik, Psi;
         if (s == 0)
             sw.first(true, zmu, chiTot, S, zz[k], chiProbe, zz[N - 2], bbc0, bbc1, Ik, Psi);
         else
             sw.step(s == N - 1, zmu, chiTot, rchi, S, zz[k], Ik, Psi);
+
+        if constexpr (DEPTH) {
+            const size_t o = (((size_t)c * N + k) * Nspect + la) * p.nmu + m;
+            if (p.dchi != nullptr) p.dchi[o] = chiTot;
+            if (p.dS != nullptr) p.dS[o] = S;
+            if (p.dI != nullptr) p.dI[o] = Ik;
+            if (p.dtau != nullptr && s > 0) p.dtau[o] = dtau;
+            // delta[k] = w0 S' + w1 dS with the w step() applied (the stale one at k = 0); delta[N-1] = the boundary I
+            if (p.dcontrib != nullptr) p.dcontrib[o] = s == 0 ? Ik : sw.w0 * Sw + sw.w1 * dS;
+        }
     }
-    p.I[((size_t)c * Nspect + la) * p.nmu + m] = sw.Iupw;   // the emergent intensity (rh_method.py:638)
+    if constexpr (!DEPTH)
+        p.I[((size_t)c * Nspect + la) * p.nmu + m] = sw.Iupw;   // the emergent intensity (rh_method.py:638)
     if (p.bad != nullptr && sw.bad()) atomicOr(p.bad + c, 2);
+
+    // ---- pass 2, top down, over what this thread stored above (plain loads of its own writes; no other thread
+    // touches these addresses)
+    if constexpr (DEPTH) {
+        if (p.dtau == nullptr) return;
+        const size_t dk = (size_t)Nspect * p.nmu;
+        double *tauk = p.dtau + ((size_t)c * N * Nspect + la) * p.nmu + m;   // depth 0 of this ray
+        double *ck = p.dcontrib == nullptr ? nullptr : p.dcontrib + (tauk - p.dtau);
+        double w0, w1;
+        w2(tauk[dk], w0, w1);           // the step into 1, whose w step() applied again at k = 0
+        double a = 1.0 - w0;            // a[0]
+        double tau = 0.0, T = 1.0, dPrev = 0.0;
+        double zt = __longlong_as_double(0x7ff8000000000000LL);   // NaN: the ray never reaches tau = 1
+        bool found = false;
+        for (int k = 0; k < N; ++k, tauk += dk) {
+            const double tauPrev = tau;
+            if (k > 0) tau = tau + dPrev;                 // tau[k] = tau[k-1] + dtau[k-1]
+            const double d = k < N - 1 ? *tauk : 0.0;     // dtau[k], read before tau[k] replaces it
+            *tauk = tau;
+            if (!found && tau >= 1.0) {
+                found = true;
+                zt = zz[k - 1] + (zz[k] - zz[k - 1]) * ((1.0 - tauPrev) / (tau - tauPrev));
+            }
+            if (ck != nullptr) {
+                *ck = *ck * T;                            // contrib[k] = delta[k] T[k]
+                ck += dk;
+            }
+            if (k > 0 && k < N - 1) {
+                w2(d, w0, w1);
+                a = 1.0 - w0;                             // a[k]
+            }
+            T = T * a;                                    // T[k+1] = T[k] a[k]
+            dPrev = d;
+        }
+        if (p.ztau1 != nullptr) p.ztau1[((size_t)c * Nspect + la) * p.nmu + m] = zt;
+    }
 }
 
 }  // namespace mali

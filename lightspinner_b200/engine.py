@@ -7,11 +7,13 @@ radiative model, and drives libmali_b200.so through its C ABI.
     dP = eng.stat_equil()                                 # [ncol] numpy   (rh_method.py:710-745)
     eng.J(col), eng.I(col), eng.Gamma(col), eng.n(col)    # numpy, reference shapes
     I = eng.compute_rays([1.0, 0.5])                      # [ncol, Nspect, nmu] emergent intensity at user angles
+    d = eng.compute_rays_depth([1.0, 0.5])                # RayDepthData: I, chi, S, tau, contrib per depth, z_tau1
 
 Columns are independent (no cross-column arithmetic anywhere), which is what makes the path data-parallel:
 ranks of a multi-GPU job each own a contiguous slice of columns (see lightspinner_b200/sharding.py).
 """
 import ctypes as C
+from dataclasses import dataclass
 
 import numpy as np
 import torch
@@ -412,12 +414,9 @@ class MaliEngine:
                                      'numeric domain in column(s) %s' % bad[:8].tolist())
 
     # ------------------------------------------------------------------ emergent intensity at user angles
-    def compute_rays_async(self, mus, col0=0, ncol=None, out=None):
-        """Emergent intensity at the angles `mus` (0 < mu <= 1; a scalar is one angle) from the current populations and
-        J of columns [col0, col0+ncol) (mali_compute_rays): a device tensor [ncol, Nspect, nmu], `out` if given.  It is
-        what the next formal solution would return as I if those angles were its quadrature angles; nothing else is
-        written, so it can be called between any two iterations.  Lists longer than MALI_RAYS_MAX_MU are split into
-        several launches.  Domain faults are collected for compute_rays (see there)."""
+    def _rays_setup(self, mus, col0, ncol):
+        """The checks compute_rays_async and compute_rays_depth_async share (the angles, the column range, every column
+        with its profile inputs); returns the angles, ncol and the profile-input pointers, and zeroes the fault words."""
         mus = rays_angles(mus)
         ncol = self.ncol - col0 if ncol is None else ncol
         if col0 < 0 or ncol < 1 or col0 + ncol > self.ncol:
@@ -426,15 +425,31 @@ class MaliEngine:
             bad = col0 + np.nonzero(~self._has_profile[col0:col0 + ncol])[0]
             raise ValueError('column(s) %s were uploaded with host line profiles and without their inputs (aDamp, vBroad, '
                              'vlos): compute_rays needs those to form the profiles at new angles' % bad[:8].tolist())
+        self._rays_bad = torch.zeros(ncol, dtype=torch.int32, device=self.device)
+        P = lambda t: C.c_void_p(t.data_ptr()) if t.numel() else None
+        return mus, ncol, [P(self.t_aDamp[col0:]), P(self.t_vBroad[col0:]), P(self.t_vlos[col0:])]
+
+    def _raise_rays_faults(self, col0):
+        bad = self._rays_bad.cpu().numpy()
+        if (bad & 2).any():
+            cols = col0 + np.nonzero(bad & 2)[0]
+            raise FloatingPointError('opacity or optical-depth step outside the formal solver\'s numeric domain '
+                                     '(zero, subnormal, infinite or NaN) in column(s) %s' % cols[:8].tolist())
+
+    def compute_rays_async(self, mus, col0=0, ncol=None, out=None):
+        """Emergent intensity at the angles `mus` (0 < mu <= 1; a scalar is one angle) from the current populations and
+        J of columns [col0, col0+ncol) (mali_compute_rays): a device tensor [ncol, Nspect, nmu], `out` if given.  It is
+        what the next formal solution would return as I if those angles were its quadrature angles; nothing else is
+        written, so it can be called between any two iterations.  Lists longer than MALI_RAYS_MAX_MU are split into
+        several launches.  Domain faults are collected for compute_rays (see there)."""
+        mus, ncol, args = self._rays_setup(mus, col0, ncol)
         nmu, S = mus.shape[0], self.mt.Nspect
         if out is None:
             out = torch.empty(ncol, S, nmu, dtype=torch.float64, device=self.device)
         elif (tuple(out.shape) != (ncol, S, nmu) or out.dtype != torch.float64 or out.device != self.device
               or not out.is_contiguous()):
             raise ValueError('out must be a contiguous float64 tensor [%d, %d, %d] on %s' % (ncol, S, nmu, self.device))
-        self._rays_bad = torch.zeros(ncol, dtype=torch.int32, device=self.device)
-        P = lambda t: C.c_void_p(t.data_ptr()) if t.numel() else None
-        args = [P(self.t_aDamp[col0:]), P(self.t_vBroad[col0:]), P(self.t_vlos[col0:])]
+        P = lambda t: C.c_void_p(t.data_ptr())
         step = _capi.RAYS_MAX_MU
         with torch.cuda.device(self.device):
             for q0 in range(0, nmu, step):
@@ -453,12 +468,75 @@ class MaliEngine:
         col0 = int(col0)
         out = self.compute_rays_async(mus, col0, ncol)
         res = out.cpu().numpy()
-        bad = self._rays_bad.cpu().numpy()
-        if (bad & 2).any():
-            cols = col0 + np.nonzero(bad & 2)[0]
-            raise FloatingPointError('opacity or optical-depth step outside the formal solver\'s numeric domain '
-                                     '(zero, subnormal, infinite or NaN) in column(s) %s' % cols[:8].tolist())
+        self._raise_rays_faults(col0)
         return res
+
+    def compute_rays_depth_async(self, mus, col0=0, ncol=None, quantities=None, out=None):
+        """Depth-resolved data of the rays compute_rays sweeps (mali_compute_rays_depth; definitions in
+        include/mali_b200.h): a dict of device tensors, one per name in `quantities` (default RAYS_DEPTH_QUANTITIES):
+        'I', 'chi', 'S', 'tau', 'contrib' [ncol, Nspace, Nspect, nmu] (depth 0 at the top), 'z_tau1' [ncol, Nspect, nmu]
+        (the height of tau = 1 along each ray, NaN if it is never reached) and 'height' [ncol, Nspace].  `out` may map
+        some of those names to contiguous float64 device tensors of those shapes to be filled.  The same checks as
+        compute_rays_async; nothing else is written.  Lists longer than MALI_RAYS_MAX_MU are split into several
+        launches.  Domain faults are collected for compute_rays_depth."""
+        want = rays_depth_quantities(quantities)
+        mus, ncol, args = self._rays_setup(mus, col0, ncol)
+        nmu, N, S = mus.shape[0], self.mt.Nspace, self.mt.Nspect
+
+        def shape(k, n):
+            return (ncol, S, n) if k == 'z_tau1' else (ncol, N) if k == 'height' else (ncol, N, S, n)
+
+        def empty(k, n):
+            return torch.empty(shape(k, n), dtype=torch.float64, device=self.device)
+
+        res = {}
+        for k, t in (out or {}).items():
+            if k not in want:
+                raise ValueError('out[%r] was given but %r is not among the requested quantities %s' % (k, k, want))
+            if (tuple(t.shape) != shape(k, nmu) or t.dtype != torch.float64 or t.device != self.device
+                    or not t.is_contiguous()):
+                raise ValueError('out[%r] must be a contiguous float64 tensor %s on %s' % (k, list(shape(k, nmu)),
+                                                                                          self.device))
+            res[k] = t
+        for k in want:
+            if k not in res:
+                res[k] = empty(k, nmu)
+        # contrib and z_tau1 are formed from the optical-depth steps the kernel keeps in the tau buffer
+        launch = list(want) + (['tau'] if 'tau' not in want and ('contrib' in want or 'z_tau1' in want) else [])
+        P = lambda t: C.c_void_p(t.data_ptr())
+        step = _capi.RAYS_MAX_MU
+        with torch.cuda.device(self.device):
+            for q0 in range(0, nmu, step):
+                part = mus[q0:q0 + step]
+                n = part.shape[0]
+                dst = {}
+                for k in launch:
+                    if k == 'height':
+                        if q0 == 0:
+                            dst[k] = res[k]
+                    else:
+                        dst[k] = res[k] if k in res and n == nmu else empty(k, n)
+                if not dst:     # only the heights were asked for, and the first launch wrote them
+                    break
+                desc = _capi.RaysDepthOut(**{k: P(t) for k, t in dst.items()})
+                self._check(self.lib.mali_compute_rays_depth(self._handle, C.byref(self.bufs), col0, ncol, n,
+                                                             part.ctypes.data_as(C.POINTER(C.c_double)), *args,
+                                                             C.byref(desc), P(self._rays_bad), self._stream()))
+                for k, t in dst.items():
+                    if k in res and t is not res[k]:
+                        res[k][..., q0:q0 + n].copy_(t)
+        return {k: res[k] for k in want}
+
+    def compute_rays_depth(self, mus, col0=0, ncol=None, quantities=None):
+        """compute_rays_depth_async as a RayDepthData of numpy arrays (the angles, the heights, and the requested
+        quantities; the others are None).  Raises FloatingPointError on a domain fault, as compute_rays does."""
+        col0 = int(col0)
+        want = rays_depth_quantities(quantities)
+        dev = self.compute_rays_depth_async(mus, col0, ncol, tuple(want) + (() if 'height' in want else ('height',)))
+        host = {k: t.cpu().numpy() for k, t in dev.items()}
+        self._raise_rays_faults(col0)
+        return RayDepthData(mu=rays_angles(mus), height=host['height'],
+                            **{k: host.get(k) for k in RAYS_DEPTH_QUANTITIES if k != 'height'})
 
     def reset_iteration_state(self):
         self.t_iter.zero_()
@@ -590,6 +668,44 @@ def rays_angles(mus):
     if not ok.all():
         raise ValueError('every mu must lie in (0, 1]: got %s' % a[~ok][:8].tolist())
     return np.ascontiguousarray(a)
+
+
+RAYS_DEPTH_QUANTITIES = ('I', 'chi', 'S', 'tau', 'contrib', 'z_tau1', 'height')
+
+
+def rays_depth_quantities(quantities):
+    """The quantities of a compute_rays_depth call as a tuple in RAYS_DEPTH_QUANTITIES order: None means all of them,
+    a string is one name; unknown names, repeats and an empty selection raise ValueError."""
+    if quantities is None:
+        return RAYS_DEPTH_QUANTITIES
+    q = [quantities] if isinstance(quantities, str) else list(quantities)
+    unknown = [k for k in q if k not in RAYS_DEPTH_QUANTITIES]
+    if unknown:
+        raise ValueError('unknown quantities %s (known: %s)' % (unknown, ', '.join(RAYS_DEPTH_QUANTITIES)))
+    if not q or len(set(q)) != len(q):
+        raise ValueError('quantities must name each of %s at most once, and at least one: got %s'
+                         % (', '.join(RAYS_DEPTH_QUANTITIES), q))
+    return tuple(k for k in RAYS_DEPTH_QUANTITIES if k in q)
+
+
+@dataclass
+class RayDepthData:
+    """Depth-resolved data of up-going rays at the angles `mu` (MaliEngine / Context / BatchContext.compute_rays_depth;
+    definitions in include/mali_b200.h).  With a leading column axis from MaliEngine and BatchContext, without it from
+    Context: I, chi, S, tau, contrib [.., Nspace, Nspect, nmu] (depth 0 at the top), z_tau1 [.., Nspect, nmu] (NaN where
+    tau = 1 is never reached), height [.., Nspace].  Quantities that were not requested are None."""
+    mu: np.ndarray
+    height: np.ndarray
+    I: np.ndarray = None
+    chi: np.ndarray = None
+    S: np.ndarray = None
+    tau: np.ndarray = None
+    contrib: np.ndarray = None
+    z_tau1: np.ndarray = None
+
+    def column(self, c):
+        """The data of column c of a batched result, without the column axis."""
+        return RayDepthData(mu=self.mu, **{k: None if v is None else v[c] for k, v in vars(self).items() if k != 'mu'})
 
 
 def piecewise_linear_1d_batch(z, muz, toFrom, bbc0, bbc1, chi, S, device=None):
