@@ -25,6 +25,7 @@
  *   (no reference counterpart; Lightweaver's compute_rays) mali_compute_rays (emergent intensity at user angles)
  *   (no reference counterpart; Lightweaver's depthData)    mali_compute_rays_depth (I, chi, S, tau, contribution
  *                                                           function, tau = 1 heights along those rays)
+ *   ComputationalTransition.Rij / .Rji (declared, never filled; Lightweaver's rates)  mali_compute_rates
  *
  * Conventions
  *   - plain C, no exceptions; every function returns 0 on success, a negative MALI_E* code on argument
@@ -288,6 +289,26 @@ typedef struct {
 int mali_compute_rays_depth(const mali_model *m, const mali_buffers *b, int32_t col0, int32_t ncol, int32_t nmu,
                             const double *mu, const double *aDamp, const double *vBroad, const double *vlos,
                             const mali_rays_depth_out *out, int32_t *bad, void *stream);
+
+/* Radiative rates of every transition from the current populations and J, columns [col0, col0+ncol) (Lightweaver's
+ * trans.Rij / trans.Rji; the reference declares the fields but never fills them).  In s^-1, like Gamma and C:
+ *   R_ij[c][t][k] = sum_{la active for t} sum_mu sum_dir  wlamu(la,mu,k) * V_ij(la,mu,dir,k) * I(la,mu,dir,k)
+ *   R_ji[c][t][k] = sum_{la active for t} sum_mu sum_dir  wlamu(la,mu,k) * (U_ji(la,mu,dir,k) + V_ji(la,mu,dir,k) * I(la,mu,dir,k))
+ *   wlamu = (wla * 0.5*wmu) * 4 pi   (wla: lines wlambda*wphi/HC, continua wlambda/lambda/h: the Gamma weights,
+ *                                     rh_method.py:451-454)
+ * over the model's quadrature angles in both directions.  I is exactly the intensity the next formal solution computes:
+ * the opacity and emissivity of the current n, the scattering term of the current J, the line profiles already in the
+ * tables, the thermalised lower boundary and the last-point quirk.  These are the Gamma integrands with PsiStar = 0;
+ * every term is non-negative wherever I is (the last-point quirk can make I, and with it R_ij, negative at the top,
+ * k = 0, on fine depth grids, exactly as in the reference's formal solution).  The net rate is n_i R_ij - n_j R_ji (m^-3 s^-1).  Always the exact arithmetic form;
+ * done is ignored (every column of the range is computed).  The partial sums are combined in a fixed order, so the
+ * result does not depend on the batch or the column range.
+ *   Rij_out, Rji_out: device [ncol][Ntrans][Nspace].  bad: device [ncol] or NULL, bit 1 as in status (the caller zeroes it).
+ * Writes Rij_out, Rji_out, bad and the Gamma-partial part of the formal-solution scratch (bufs->scratch, which holds
+ * nothing between calls); nothing else.  A model without transitions writes nothing (its outputs may be NULL).
+ * MALI_EINVAL for a bad range or a null colconst / pops / J / scratch / output. */
+int mali_compute_rates(const mali_model *m, const mali_buffers *b, int32_t col0, int32_t ncol,
+                       double *Rij_out, double *Rji_out, int32_t *bad, void *stream);
 
 /* Context.formal_sol_gamma_matrices for columns [col0, col0+ncol): updates J, I, Gamma and dJ.  J-dagger (the
  * previous call's J; zero after an upload, rh_method.py:541) is kept by the library inside colconst.  Work is

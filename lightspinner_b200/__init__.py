@@ -4,19 +4,21 @@
     from lightspinner_b200 import MaliEngine                        # batched columns on one GPU
     from lightspinner_b200 import NgOptions                         # opt-in Ng acceleration (ng=NgOptions())
     from lightspinner_b200 import RayDepthData                      # what compute_rays_depth returns
+    from lightspinner_b200 import RadiativeRates                    # what compute_rates returns
 
 The compute lives in csrc/ (hand-written CUDA for sm_100a behind the C ABI of include/mali_b200.h); there is no CPU
 fallback.  Importing the package does not touch the GPU; constructing a Context / MaliEngine does.
 """
 
-__all__ = ['Context', 'BatchContext', 'piecewise_linear_1d', 'IPsi', 'UV', 'MaliEngine', 'NgOptions', 'RayDepthData']
+__all__ = ['Context', 'BatchContext', 'piecewise_linear_1d', 'IPsi', 'UV', 'MaliEngine', 'NgOptions', 'RayDepthData',
+           'RadiativeRates']
 
 
 def __getattr__(name):
     if name in ('Context', 'BatchContext', 'piecewise_linear_1d', 'IPsi', 'UV'):
         from . import context
         return getattr(context, name)
-    if name in ('MaliEngine', 'RayDepthData'):
+    if name in ('MaliEngine', 'RayDepthData', 'RadiativeRates'):
         from . import engine
         return getattr(engine, name)
     if name == 'NgOptions':

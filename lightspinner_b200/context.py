@@ -7,6 +7,7 @@
     ctx.I, ctx.J, ctx.activeAtoms[0].n, .Gamma        # same names, shapes and aliasing as the reference
     I = ctx.compute_rays([1.0, 0.5])                  # [Nspect, nmu]: emergent intensity at user angles (Lightweaver)
     d = ctx.compute_rays_depth([1.0, 0.5])            # RayDepthData: I, chi, S, tau, contrib [Nspace, Nspect, nmu], ...
+    r = ctx.compute_rates()                           # RadiativeRates: Rij, Rji, net [Ntrans, Nspace]; fills trans.Rij/Rji
 
 Only the hot path moves to the GPU.  Everything in this file is the host-side mirror of the reference's per-Context
 SET-UP (ComputationalTransition / ComputationalAtom construction, rh_method.py:93-131,366-423,474-487): it asks the
@@ -62,7 +63,7 @@ class ComputationalTransition:
             if trans in s:
                 self.active[la] = True
         self.gij = None
-        self.Rij = np.zeros(atmos.Nspace)    # dead outputs of the reference (never zeroed, never read): not maintained
+        self.Rij = np.zeros(atmos.Nspace)    # radiative rates (s^-1), filled by Context.compute_rates (zeros until then)
         self.Rji = np.zeros(atmos.Nspace)
         self.index = None                    # position in the flattened transition table
         self._profile = None
@@ -219,6 +220,22 @@ class Context:
         self._push_pops()
         return self._engine.compute_rays_depth(mus, self._col, 1, quantities).column(0)
 
+    def compute_rates(self):
+        """Radiative rates of every transition from the current populations (edits through the eqPops alias included)
+        and the current J: a RadiativeRates with Rij, Rji (s^-1) and net (m^-3 s^-1) [Ntrans, Nspace] in the model's
+        transition order (see MaliEngine.compute_rates).  Also fills trans.Rij / trans.Rji of every
+        ComputationalTransition.  It changes nothing the iteration uses."""
+        self._push_pops()
+        r = self._engine.compute_rates(self._col, 1).column(0)
+        self._fill_rates(r)
+        return r
+
+    def _fill_rates(self, r):
+        for atom in self.activeAtoms:
+            for t in atom.trans:
+                t.Rij[...] = r.Rij[t.index]
+                t.Rji[...] = r.Rji[t.index]
+
     def ng_reset(self):
         """Restart the Ng history (Context(ng=...)): call it after editing populations between iterations."""
         self._engine.ng_reset(self._col, 1)
@@ -301,6 +318,16 @@ class BatchContext:
         for c in self.contexts:
             c._push_pops()
         return self._engine.compute_rays_depth(mus, quantities=quantities)
+
+    def compute_rates(self):
+        """Context.compute_rates for every column: a RadiativeRates with a leading column axis; fills each column's
+        trans.Rij / trans.Rji as well."""
+        for c in self.contexts:
+            c._push_pops()
+        r = self._engine.compute_rates()
+        for k, c in enumerate(self.contexts):
+            c._fill_rates(r.column(k))
+        return r
 
     def iterate(self, max_iter=500, tolJ=2e-3, tolPops=1e-3):
         """The loop of test.py:20-29 for every column, kept on the device (mali_iterate): returns the iteration

@@ -16,6 +16,7 @@
 #include "../../include/mali_b200.h"
 #include "mali_kernels.cuh"
 #include "mali_rays.cuh"
+#include "mali_rates.cuh"
 #include "mali_fs_launch.h"
 
 using namespace mali;
@@ -1136,6 +1137,57 @@ int mali_compute_rays_depth(const mali_model *m, const mali_buffers *b, int32_t 
     p.dcontrib = out->contrib;
     p.ztau1 = out->z_tau1;
     return launch_rays(m, p, true, stream);
+}
+
+int mali_compute_rates(const mali_model *m, const mali_buffers *b, int32_t col0, int32_t ncol, double *Rij_out,
+                       double *Rji_out, int32_t *bad, void *stream)
+{
+    if (int r = check_range(m, b, col0, ncol, "mali_compute_rates")) return r;
+    if (!b->colconst || !b->pops || !b->J || !b->scratch) return fail(MALI_EINVAL, "mali_compute_rates: null buffer");
+    if (m->Ntrans == 0) return MALI_OK;   // empty outputs (which may be null): nothing to write
+    if (!Rij_out || !Rji_out) return fail(MALI_EINVAL, "mali_compute_rates: null output");
+    RatesParams p{};
+    p.N = m->N;
+    p.Nrays = m->Nrays;
+    p.Nspect = m->Nspect;
+    p.Lw = m->Lw;
+    p.ntile = m->ntile;
+    p.Ntrans = m->Ntrans;
+    p.col0 = col0;
+    p.ncol = ncol;
+    p.colStride = m->lay.colconst;
+    p.popStride = m->lay.pops;
+    p.JStride = m->lay.J;
+    p.scratchStride = m->lay.scratch;
+    p.off_z = m->off_z;
+    p.off_bbc = m->off_bbc;
+    p.off_tab = m->off_tab;
+    p.off_part = m->off_part;
+    p.upOff = m->upOff;
+    p.tiles = m->d_tiles;
+    p.slots = m->d_slots;
+    p.alpha = m->d_alpha;
+    p.twohc = m->d_twohc;
+    p.wlacont = m->d_wlacont;
+    p.zmu = m->d_zmu;
+    p.hw = m->d_hw;
+    p.colconst = b->colconst;
+    p.pops = b->pops;
+    p.J = b->J;
+    p.scratch = b->scratch;
+    p.trPartOff = m->d_trPartOff;
+    p.trPartRows = m->d_trPartRows;
+    p.Rij = Rij_out;
+    p.Rji = Rji_out;
+    p.bad = bad;
+    const cudaStream_t st = (cudaStream_t)stream;
+    const int64_t warps = (int64_t)ncol * m->ntile * 2;
+    const int wpb = 4;
+    rates_kernel<<<(unsigned)((warps + wpb - 1) / wpb), 32 * wpb, 0, st>>>(p);
+    rates_finish_kernel<<<dim3((m->N + 127) / 128, m->Ntrans, ncol), 128, 0, st>>>(p);
+    m->launches += 2;
+    CU(cudaGetLastError());
+    return MALI_OK;
 }
 
 static FsParams make_fs_params(const mali_model *m, const mali_buffers *b, int col0, int ncol, int wpb)

@@ -8,6 +8,7 @@ radiative model, and drives libmali_b200.so through its C ABI.
     eng.J(col), eng.I(col), eng.Gamma(col), eng.n(col)    # numpy, reference shapes
     I = eng.compute_rays([1.0, 0.5])                      # [ncol, Nspect, nmu] emergent intensity at user angles
     d = eng.compute_rays_depth([1.0, 0.5])                # RayDepthData: I, chi, S, tau, contrib per depth, z_tau1
+    r = eng.compute_rates()                               # RadiativeRates: Rij, Rji, net [ncol, Ntrans, Nspace]
 
 Columns are independent (no cross-column arithmetic anywhere), which is what makes the path data-parallel:
 ranks of a multi-GPU job each own a contiguous slice of columns (see lightspinner_b200/sharding.py).
@@ -538,6 +539,49 @@ class MaliEngine:
         return RayDepthData(mu=rays_angles(mus), height=host['height'],
                             **{k: host.get(k) for k in RAYS_DEPTH_QUANTITIES if k != 'height'})
 
+    # ------------------------------------------------------------------ radiative rates
+    def compute_rates_async(self, col0=0, ncol=None, out=None):
+        """Radiative rates R_ij, R_ji (s^-1) of every transition from the current populations and J of columns
+        [col0, col0+ncol) (mali_compute_rates; definition in include/mali_b200.h): a pair of device tensors
+        [ncol, Ntrans, Nspace], `out` (a pair of contiguous float64 tensors of that shape) if given.  The intensity is
+        the one the next formal solution computes, with the line profiles already in the tables, so columns uploaded
+        with host profiles are served too.  The call overwrites the formal-solution scratch (which holds nothing
+        between calls) and nothing else the iteration uses.  Domain faults are collected for compute_rates."""
+        ncol = self.ncol - col0 if ncol is None else ncol
+        if col0 < 0 or ncol < 1 or col0 + ncol > self.ncol:
+            raise ValueError('columns [%d, %d) outside the batch of %d' % (col0, col0 + ncol, self.ncol))
+        shape = (ncol, self.mt.Ntrans, self.mt.Nspace)
+        if out is None:
+            out = tuple(torch.empty(shape, dtype=torch.float64, device=self.device) for _ in range(2))
+        elif (not isinstance(out, (tuple, list)) or len(out) != 2
+              or any(not isinstance(t, torch.Tensor) or tuple(t.shape) != shape or t.dtype != torch.float64
+                     or t.device != self.device or not t.is_contiguous() for t in out)):
+            raise ValueError('out must be a pair (Rij, Rji) of contiguous float64 tensors %s on %s'
+                             % (list(shape), self.device))
+        self._rays_bad = torch.zeros(ncol, dtype=torch.int32, device=self.device)
+        P = lambda t: C.c_void_p(t.data_ptr())
+        with torch.cuda.device(self.device):
+            self._check(self.lib.mali_compute_rates(self._handle, C.byref(self.bufs), col0, ncol, P(out[0]), P(out[1]),
+                                                    P(self._rays_bad), self._stream()))
+        return out[0], out[1]
+
+    def compute_rates(self, col0=0, ncol=None):
+        """compute_rates_async as a RadiativeRates of numpy arrays [ncol, Ntrans, Nspace], with the net radiative rates
+        n_i R_ij - n_j R_ji (m^-3 s^-1) from the same populations.  Raises FloatingPointError on a domain fault, as
+        compute_rays does."""
+        col0 = int(col0)
+        Rij, Rji = self.compute_rates_async(col0, ncol)
+        ncol = Rij.shape[0]
+        L = self.lay.pops
+        n = self.t_pops[col0 * L:(col0 + ncol) * L].view(ncol, -1, self.mt.Nspace)
+        tr = self.mt.trans
+        rowI = torch.as_tensor(self.mt.lvloff[tr[:, 0]] + tr[:, 1], dtype=torch.int64, device=self.device)
+        rowJ = torch.as_tensor(self.mt.lvloff[tr[:, 0]] + tr[:, 2], dtype=torch.int64, device=self.device)
+        net = n[:, rowI] * Rij - n[:, rowJ] * Rji
+        res = RadiativeRates(Rij=Rij.cpu().numpy(), Rji=Rji.cpu().numpy(), net=net.cpu().numpy())
+        self._raise_rays_faults(col0)
+        return res
+
     def reset_iteration_state(self):
         self.t_iter.zero_()
         self.t_done.zero_()
@@ -706,6 +750,20 @@ class RayDepthData:
     def column(self, c):
         """The data of column c of a batched result, without the column axis."""
         return RayDepthData(mu=self.mu, **{k: None if v is None else v[c] for k, v in vars(self).items() if k != 'mu'})
+
+
+@dataclass
+class RadiativeRates:
+    """Radiative rates of every transition (MaliEngine / Context / BatchContext.compute_rates; definition in
+    include/mali_b200.h): Rij, Rji (s^-1) and net = n_i Rij - n_j Rji (m^-3 s^-1), [.., Ntrans, Nspace] in the model's
+    transition order, with a leading column axis from MaliEngine and BatchContext, without it from Context."""
+    Rij: np.ndarray
+    Rji: np.ndarray
+    net: np.ndarray
+
+    def column(self, c):
+        """The rates of column c of a batched result, without the column axis."""
+        return RadiativeRates(Rij=self.Rij[c], Rji=self.Rji[c], net=self.net[c])
 
 
 def piecewise_linear_1d_batch(z, muz, toFrom, bbc0, bbc1, chi, S, device=None):
