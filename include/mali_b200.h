@@ -26,6 +26,7 @@
  *   (no reference counterpart; Lightweaver's depthData)    mali_compute_rays_depth (I, chi, S, tau, contribution
  *                                                           function, tau = 1 heights along those rays)
  *   ComputationalTransition.Rij / .Rji (declared, never filled; Lightweaver's rates)  mali_compute_rates
+ *   response_fn.py:23-39 (the perturbed columns of a response function)   mali_perturb_columns (one depth re-formed per column)
  *
  * Conventions
  *   - plain C, no exceptions; every function returns 0 on success, a negative MALI_E* code on argument
@@ -244,6 +245,44 @@ int mali_setup_columns(const mali_model *m, const mali_buffers *bufs, int32_t co
  * calls, is good to ~1e-13, so profiles agree with the reference's to that level, not bit for bit). */
 int mali_compute_phi(const mali_model *m, const mali_buffers *bufs, int32_t col0, int32_t ncol, const double *aDamp,
                      const double *vBroad, const double *vlos, void *stream);
+
+/* Columns that differ from one set-up column at a single depth each (the columns of a response function,
+ * response_fn.py): column col0 + c becomes the source column src_col with depth depth[c] re-formed from the column's own
+ * inputs, without re-forming its other depths.
+ *   1. Clone: the source's colconst block (heights, boundary Planck pair, C, nTotal, tables), its EOS work rows, nStar
+ *      and vBroad are copied to every column of the range; J is zeroed and the populations are set to pops0.  The source
+ *      must have been set up (mali_upload_columns_thermo + mali_background + mali_setup_columns + mali_compute_phi) and
+ *      never iterated, so that the J-dagger fields of its records are zero.
+ *   2. Depth depth[c] of each column is re-formed with the device arithmetic of the full set-up: the EOS point, the
+ *      background fields at every wavelength, LTE populations, C and vBroad, the continua's g_ij and continuum-group
+ *      fields, and the line profiles, Vij rows and weight fields.  The whole depth is re-formed whatever input changed.
+ *   3. Heights: with cmass, convert_scales' column-mass recurrence runs over the range on the clone's EOS work rows with
+ *      row depth[c] replaced; without, the source's heights stay.  Where bbc is given it replaces the boundary Planck pair.
+ * Afterwards each column holds bit for bit what the full set-up (with pops0 as the starting populations) produces from
+ * its inputs -- colconst, J, nStar and vBroad -- provided those inputs differ from the source's only at depth[c] (and
+ * bbc, where given, is the pair mali_planck_bc forms from the column's temperature).
+ * The depths travel to the device through a buffer the model owns: calls on one model must not overlap in time on
+ * different streams.
+ * MALI_EINVAL for a bad range, a source column outside the batch or inside the range, a depth outside [0, Nspace), a
+ * null required pointer, and when mali_model_set_eos / mali_model_set_atoms (or, for a model with lines,
+ * mali_model_desc.lambda0) are missing. */
+typedef struct {
+    const int32_t *depth;      /* HOST [ncol]: the re-formed depth of each column, 0 <= depth < Nspace */
+    const double *T, *ne, *nHTot, *vturb, *vlos;   /* device [ncol][Nspace]: the columns' full inputs */
+    const double *cmass;       /* device [ncol][Nspace] column mass (the source's depth scale), or NULL: heights kept */
+    const double *aDamp;       /* device [ncol][Ntrans][Nspace] */
+    const double *bbc;         /* device [ncol][Nspect][2] boundary Planck pairs, or NULL: the source's are kept */
+    const double *pops0;       /* device [sumNlevel][Nspace]: the populations every column starts from */
+    const double *src_work;    /* device [Nspace][20]: the first ncol*Nspace*20 doubles mali_background left in its work
+                                  buffer for a call whose only column was the source */
+    const double *src_nStar;   /* device [sumNlevel][Nspace], src_vBroad [Natom][Nspace]: the source's mali_setup_columns */
+    const double *src_vBroad;  /*   outputs */
+    double *work;              /* device scratch of ncol * Nspace * 21 doubles */
+    double *nStar;             /* device [ncol][sumNlevel][Nspace] out */
+    double *vBroad;            /* device [ncol][Natom][Nspace] out */
+} mali_perturb_desc;
+int mali_perturb_columns(const mali_model *m, const mali_buffers *bufs, int32_t src_col, int32_t col0, int32_t ncol,
+                         const mali_perturb_desc *d, void *stream);
 
 /* Emergent intensity at user angles from the current populations and J, for columns [col0, col0+ncol) (Lightweaver's
  * Context.compute_rays; the reference has no counterpart).  I_out[c][la][m] is what the NEXT mali_formal_sol_gamma would

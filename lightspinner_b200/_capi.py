@@ -55,6 +55,12 @@ class RaysDepthOut(C.Structure):
     _fields_ = [(n, C.c_void_p) for n in ('I', 'chi', 'S', 'tau', 'contrib', 'z_tau1', 'height')]
 
 
+class PerturbDesc(C.Structure):
+    _fields_ = [('depth', _ip)] + [(n, C.c_void_p) for n in (
+        'T', 'ne', 'nHTot', 'vturb', 'vlos', 'cmass', 'aDamp', 'bbc', 'pops0', 'src_work', 'src_nStar', 'src_vBroad',
+        'work', 'nStar', 'vBroad')]
+
+
 class NgParams(C.Structure):
     _fields_ = [('order', C.c_int32), ('delay', C.c_int32), ('period', C.c_int32)]
 
@@ -70,7 +76,7 @@ EXPORTS = ['mali_last_error', 'mali_device_count', 'mali_model_create', 'mali_mo
            'mali_upload_columns_atmos', 'mali_model_set_atoms', 'mali_setup_columns',
            'mali_upload_columns_thermo', 'mali_model_set_eos', 'mali_background', 'mali_graph_iterations',
            'mali_ng_layout', 'mali_stat_equil_ng', 'mali_iterate_ng', 'mali_ng_hook', 'mali_compute_rays',
-           'mali_compute_rays_depth', 'mali_compute_rates']
+           'mali_compute_rays_depth', 'mali_compute_rates', 'mali_perturb_columns']
 
 RAYS_MAX_MU = 64   # MALI_RAYS_MAX_MU
 
@@ -137,6 +143,8 @@ def load(path=None):
     L.mali_compute_rays_depth.argtypes = [C.c_void_p, C.POINTER(Buffers), C.c_int32, C.c_int32, C.c_int32, _dp] + \
         [C.c_void_p] * 3 + [C.POINTER(RaysDepthOut), C.c_void_p, C.c_void_p]
     L.mali_compute_rates.argtypes = [C.c_void_p, C.POINTER(Buffers), C.c_int32, C.c_int32] + [C.c_void_p] * 4
+    L.mali_perturb_columns.argtypes = [C.c_void_p, C.POINTER(Buffers), C.c_int32, C.c_int32, C.c_int32,
+                                       C.POINTER(PerturbDesc), C.c_void_p]
     L.mali_uv.argtypes = [C.c_void_p, C.POINTER(Buffers)] + [C.c_int32] * 5 + [C.c_void_p] * 4
     _libs[path] = L
     return L

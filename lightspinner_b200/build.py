@@ -22,14 +22,16 @@ CHECK_LIB = os.path.join(LIBDIR, 'libmali_b200_check.so')
 CHECK_DEFINES = ['MALI_CHECK=1']
 DEPS = ['mali_api.cu', 'mali_fs_class.cu', 'mali_fs_launch.h', 'mali_kernels.cuh', 'mali_device.cuh', 'mali_types.cuh',
         'exp_table.inc', 'mali_solve.h', 'mali_voigt.h', 'mali_fs_spec.cuh', 'mali_fs_step.inc', 'spec_instances.inc',
-        'mali_rays.cuh', 'mali_rates.cuh', os.path.join('..', '..', 'include', 'mali_b200.h')]
+        'mali_rays.cuh', 'mali_rates.cuh', 'mali_perturb.cuh', 'mali_eos.h', 'mali_eos_tables.inc',
+        os.path.join('..', '..', 'include', 'mali_b200.h')]
 
 EXTRA = os.environ.get('MALI_NVCC_EXTRA', '').split()
 NVCC_FLAGS = EXTRA + ['-gencode', 'arch=compute_100a,code=sm_100a', '-O3', '-lineinfo', '--fmad=false', '-std=c++20',
                       '-Xcompiler', '-fPIC', '-Xcompiler', '-ffp-contract=off', '-Xcompiler', '-O2']
 # (mali_voigt.h is reached by every unit through mali_device.cuh, but only compute_phi_kernel in mali_kernels.cuh and
 # rays_kernel in mali_rays.cuh call it)
-API_ONLY = {'mali_api.cu', 'mali_kernels.cuh', 'mali_rays.cuh', 'mali_rates.cuh', 'mali_voigt.h', os.path.join('..', '..', 'include', 'mali_b200.h')}
+API_ONLY = {'mali_api.cu', 'mali_kernels.cuh', 'mali_rays.cuh', 'mali_rates.cuh', 'mali_perturb.cuh', 'mali_eos.h',
+            'mali_eos_tables.inc', 'mali_voigt.h', os.path.join('..', '..', 'include', 'mali_b200.h')}
 FS_ONLY = {'mali_fs_class.cu', 'mali_fs_step.inc', 'spec_instances.inc'}
 # (object name, source, extra flags)
 UNITS = [('fs1', 'mali_fs_class.cu', ['-DMALI_CLS=1']), ('fs1f', 'mali_fs_class.cu', ['-DMALI_CLS=1', '-DMALI_FAST=1']),

@@ -17,6 +17,7 @@
 #include "mali_kernels.cuh"
 #include "mali_rays.cuh"
 #include "mali_rates.cuh"
+#include "mali_perturb.cuh"
 #include "mali_fs_launch.h"
 
 using namespace mali;
@@ -223,6 +224,8 @@ struct mali_model {
     mutable int profUsed = 0;
     mutable bool profOn = false;
     mutable long long launches = 0;  // kernels launched through this model since creation
+    mutable int32_t *d_depth = nullptr;  // mali_perturb_columns' depth list on the device
+    mutable int depthCap = 0;
 };
 
 extern "C" {
@@ -749,6 +752,7 @@ void mali_model_destroy(mali_model *m)
         if (p) cudaFree(p);
     for (void *p : m->eosDev)
         if (p) cudaFree(p);
+    if (m->d_depth) cudaFree(m->d_depth);
     for (auto &g : m->iterGraphs) cudaGraphExecDestroy(g.exec);
     for (cudaEvent_t e : m->profEvents) cudaEventDestroy(e);
     for (int q = 0; q < 2; ++q) {
@@ -1034,6 +1038,95 @@ int mali_compute_phi(const mali_model *m, const mali_buffers *b, int32_t col0, i
         m->N, m->Nrays, m->Nspect, m->Lw, m->Ntrans, m->Natom, aDamp, vBroad, vlos, b->colconst, m->lay.colconst, m->off_tab,
         col0);
     m->launches += 1;
+    CU(cudaGetLastError());
+    return MALI_OK;
+}
+
+int mali_perturb_columns(const mali_model *m, const mali_buffers *b, int32_t src_col, int32_t col0, int32_t ncol,
+                         const mali_perturb_desc *d, void *stream)
+{
+    if (int r = check_range(m, b, col0, ncol, "mali_perturb_columns")) return r;
+    if (src_col < 0 || src_col >= b->ncol) return fail(MALI_EINVAL, "mali_perturb_columns: source column %d outside the batch of %d", src_col, b->ncol);
+    if (src_col >= col0 && src_col < col0 + ncol)
+        return fail(MALI_EINVAL, "mali_perturb_columns: source column %d inside the range [%d, %d)", src_col, col0, col0 + ncol);
+    if (!d || !d->depth || !d->T || !d->ne || !d->nHTot || !d->vturb || !d->vlos || !d->aDamp || !d->pops0 || !d->src_work ||
+        !d->src_nStar || !d->src_vBroad || !d->work || !d->nStar || !d->vBroad || !b->colconst || !b->pops || !b->J)
+        return fail(MALI_EINVAL, "mali_perturb_columns: null argument");
+    if (!m->haveEos || !m->haveAtoms) return fail(MALI_EINVAL, "mali_perturb_columns: call mali_model_set_eos and mali_model_set_atoms first");
+    if (m->nPhiLines > 0 && !m->haveLambda0) return fail(MALI_EINVAL, "mali_perturb_columns: the model was created without lambda0");
+    for (int c = 0; c < ncol; ++c)
+        if (d->depth[c] < 0 || d->depth[c] >= m->N)
+            return fail(MALI_EINVAL, "mali_perturb_columns: depth[%d]=%d not in [0, %d)", c, d->depth[c], m->N);
+    cudaStream_t st = (cudaStream_t)stream;
+    if (ncol > m->depthCap) {
+        if (m->d_depth) CU(cudaFree(m->d_depth));
+        m->d_depth = nullptr;
+        m->depthCap = 0;
+        CU(cudaMalloc((void **)&m->d_depth, (size_t)ncol * sizeof(int32_t)));
+        m->depthCap = ncol;
+    }
+    CU(cudaMemcpyAsync(m->d_depth, d->depth, (size_t)ncol * sizeof(int32_t), cudaMemcpyHostToDevice, st));
+    PerturbParams p{};
+    p.N = m->N;
+    p.Nspect = m->Nspect;
+    p.Lw = m->Lw;
+    p.sumNlevel = m->sumNlevel;
+    p.Natom = m->Natom;
+    p.col0 = col0;
+    p.src = src_col;
+    p.colStride = m->lay.colconst;
+    p.popStride = m->lay.pops;
+    p.JStride = m->lay.J;
+    p.off_bbc = m->off_bbc;
+    p.off_tab = m->off_tab;
+    p.depth = m->d_depth;
+    p.T = d->T;
+    p.ne = d->ne;
+    p.nHTot = d->nHTot;
+    p.vturb = d->vturb;
+    p.bbc = d->bbc;
+    p.pops0 = d->pops0;
+    p.srcWork = d->src_work;
+    p.srcNStar = d->src_nStar;
+    p.srcVBroad = d->src_vBroad;
+    p.work = d->work;
+    p.nStar = d->nStar;
+    p.vBroad = d->vBroad;
+    p.colconst = b->colconst;
+    p.pops = b->pops;
+    p.J = b->J;
+    // 1. clone
+    const int nb = (int)std::min<int64_t>(64, (m->lay.colconst / 2 + 255) / 256);
+    perturb_clone_kernel<<<dim3(nb, ncol), 256, 0, st>>>(p);
+    // 2. re-form depth[c]: EOS point, then background and levels (both read it), then g_ij, groups and profiles
+    perturb_eos_kernel<<<(ncol + 63) / 64, 64, 0, st>>>(m->eos, p, ncol);
+    perturb_background_kernel<<<dim3((m->Nspect + 63) / 64, ncol), 64, 0, st>>>(m->eos, m->d_tiles, m->d_wavelength, d->ne, p);
+    const int na = ncol * m->Natom;
+    if (m->maxNlevel <= 8)
+        perturb_levels_kernel<8><<<(na + 63) / 64, 64, 0, st>>>(m->atoms, p, m->off_C, m->off_nTotal, ncol);
+    else
+        perturb_levels_kernel<16><<<(na + 63) / 64, 64, 0, st>>>(m->atoms, p, m->off_C, m->off_nTotal, ncol);
+    m->launches += 4;
+    if (m->nGijCont > 0) {
+        perturb_gij_kernel<<<dim3(m->nGijCont, ncol), 64, 0, st>>>(m->d_gijCont, m->d_gijTiles, m->d_wavelength, m->d_alpha, p);
+        m->launches += 1;
+        if (m->nGroupTiles > 0) {
+            perturb_group_kernel<<<dim3(m->nGroupTiles, ncol), m->Lw, 0, st>>>(m->d_tiles, m->d_slots, m->d_groupTiles, m->d_twohc, p);
+            m->launches += 1;
+        }
+    }
+    if (m->nPhiLines > 0) {
+        perturb_phi_kernel<<<dim3(m->nPhiLines, ncol), 32, 0, st>>>(m->d_phiLines, m->d_phiTiles, m->d_wavelength, m->d_wlambda,
+                                                                     m->d_muz, m->d_wmu, m->Nrays, m->Ntrans, d->aDamp, d->vlos, p);
+        m->launches += 1;
+    }
+    // 3. heights from the column mass over the whole range (the recurrence is not local in depth)
+    if (d->cmass) {
+        double *tau = d->work + (size_t)ncol * m->N * kEosWork;
+        convert_scales_kernel<<<(ncol + 31) / 32, 32, 0, st>>>(m->eos, m->N, ncol, d->cmass, d->nHTot, d->work, b->colconst,
+                                                               m->lay.colconst, m->off_z, col0, tau);
+        m->launches += 1;
+    }
     CU(cudaGetLastError());
     return MALI_OK;
 }

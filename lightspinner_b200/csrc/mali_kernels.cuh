@@ -741,6 +741,51 @@ struct PhiLine {
 struct PhiTile {
     int32_t v0, vDir, f, stride;   // depth-0 offsets of the line's direction-0 Vij row and of its weight field; distance
 };                                 // to the direction-1 row; record stride of the tile
+// The body of compute_phi_kernel from the line, depth and column on (`ln`, `k`, `c`, `lane` and the kernel's parameters
+// in scope), shared with the depth re-formation of mali_perturb_columns (mali_perturb.cuh).  A macro rather than an
+// inlined function: every function form of it changed the instruction order of the kernel (the loop over the weight
+// fields), whose SASS is kept byte for byte.
+#define MALI_COMPUTE_PHI_BODY()                                                                                       \
+    do {                                                                                                              \
+    const double ad = aDamp[((size_t)c * Ntrans + ln.t) * N + k];                                                     \
+    const double vb = vBroad[((size_t)c * Natom + ln.atom) * N + k];                                                  \
+    const double vl = vlos[(size_t)c * N + k];                                                                        \
+    double *tab = colconst + (size_t)(col0 + c) * colStride + offTab;                                                 \
+    const int ls = lane / Nrays, mu = lane - ls * Nrays;                                                              \
+    const bool lane_on = ls < Lw;                                                                                     \
+    const double sqrtPi = sqrt(kPi);                                                                                  \
+    const double rnorm = 1.0 / (sqrtPi * vb);                                                                         \
+    const VoigtPre vp = voigt_pre(ad);   /* the damping-only part of the Voigt evaluation, once per (line, depth) */  \
+    const double vd = lane_on ? muz[mu] * vl / vb : 0.0;   /* :223 */                                                 \
+    const double wm = lane_on ? wmu[mu] : 0.0;                                                                        \
+    double wPhi = 0.0;                                                                                                \
+    for (int j = 0; j < ln.ntile; ++j) {                                                                              \
+        const int la = (ln.tile0 + j) * Lw + ls, lt = la - ln.Nblue;                                                  \
+        const bool on = lane_on && lt >= 0 && lt < ln.Nlam && la < Nspect;                                            \
+        double p0 = 0.0, p1 = 0.0;                                                                                    \
+        if (on) {                                                                                                     \
+            const double v = (wavelength[la] - ln.lambda0) * kCLight / (vb * ln.lambda0);   /* :225 */                \
+            p0 = voigt_H_pre(vp, v - vd) * rnorm;   /* :229-231 */                                                    \
+            p1 = voigt_H_pre(vp, v + vd) * rnorm;                                                                     \
+            wPhi += (p0 + p1) * ((wlambda[ln.toff + lt] * 0.5) * wm);   /* :227, :233 */                              \
+        }                                                                                                             \
+        const PhiTile pt = ptile[ln.tab0 + j];                                                                        \
+        double *v0 = tab + pt.v0 + (size_t)k * pt.stride;                                                             \
+        v0[lane] = ln.c0 * p0;   /* whole rows, zero where the line is not active */                                  \
+        v0[pt.vDir + lane] = ln.c0 * p1;                                                                              \
+    }                                                                                                                 \
+    _Pragma("unroll")                                                                                                 \
+    for (int off = 16; off > 0; off >>= 1) wPhi += __shfl_xor_sync(0xffffffffu, wPhi, off);                           \
+    const double wphi = 1.0 / wPhi;   /* :235 */                                                                      \
+    for (int j = 0; j < ln.ntile; ++j) {                                                                              \
+        if (lane < Lw) {                                                                                              \
+            const int la = (ln.tile0 + j) * Lw + lane, lt = la - ln.Nblue;                                            \
+            const bool on = lt >= 0 && lt < ln.Nlam && la < Nspect;                                                   \
+            const PhiTile pt = ptile[ln.tab0 + j];                                                                    \
+            tab[pt.f + (size_t)k * pt.stride + lane] = on ? wlambda[ln.toff + lt] * wphi / kHC : 0.0;   /* :451 */    \
+        }                                                                                                             \
+    }                                                                                                                 \
+    } while (0)
 __global__ void compute_phi_kernel(const PhiLine *lines, const PhiTile *ptile, const double *wavelength, const double *wlambda,
                                    const double *muz, const double *wmu, int N, int Nrays, int Nspect, int Lw, int Ntrans,
                                    int Natom, const double *aDamp, const double *vBroad, const double *vlos,
@@ -751,44 +796,7 @@ __global__ void compute_phi_kernel(const PhiLine *lines, const PhiTile *ptile, c
     if (k >= N) return;
     const PhiLine ln = lines[blockIdx.y];
     const int c = blockIdx.z;                      // column inside the call's inputs
-    const double ad = aDamp[((size_t)c * Ntrans + ln.t) * N + k];
-    const double vb = vBroad[((size_t)c * Natom + ln.atom) * N + k];
-    const double vl = vlos[(size_t)c * N + k];
-    double *tab = colconst + (size_t)(col0 + c) * colStride + offTab;
-    const int ls = lane / Nrays, mu = lane - ls * Nrays;
-    const bool lane_on = ls < Lw;
-    const double sqrtPi = sqrt(kPi);
-    const double rnorm = 1.0 / (sqrtPi * vb);
-    const VoigtPre vp = voigt_pre(ad);             // the damping-only part of the Voigt evaluation, once per (line, depth)
-    const double vd = lane_on ? muz[mu] * vl / vb : 0.0;                                        // :223
-    const double wm = lane_on ? wmu[mu] : 0.0;
-    double wPhi = 0.0;
-    for (int j = 0; j < ln.ntile; ++j) {
-        const int la = (ln.tile0 + j) * Lw + ls, lt = la - ln.Nblue;
-        const bool on = lane_on && lt >= 0 && lt < ln.Nlam && la < Nspect;
-        double p0 = 0.0, p1 = 0.0;
-        if (on) {
-            const double v = (wavelength[la] - ln.lambda0) * kCLight / (vb * ln.lambda0);      // :225
-            p0 = voigt_H_pre(vp, v - vd) * rnorm;                                               // :229-231
-            p1 = voigt_H_pre(vp, v + vd) * rnorm;
-            wPhi += (p0 + p1) * ((wlambda[ln.toff + lt] * 0.5) * wm);                           // :227, :233
-        }
-        const PhiTile pt = ptile[ln.tab0 + j];
-        double *v0 = tab + pt.v0 + (size_t)k * pt.stride;
-        v0[lane] = ln.c0 * p0;                         // whole rows, zero where the line is not active
-        v0[pt.vDir + lane] = ln.c0 * p1;
-    }
-#pragma unroll
-    for (int off = 16; off > 0; off >>= 1) wPhi += __shfl_xor_sync(0xffffffffu, wPhi, off);
-    const double wphi = 1.0 / wPhi;                                                             // :235
-    for (int j = 0; j < ln.ntile; ++j) {
-        if (lane < Lw) {
-            const int la = (ln.tile0 + j) * Lw + lane, lt = la - ln.Nblue;
-            const bool on = lt >= 0 && lt < ln.Nlam && la < Nspect;
-            const PhiTile pt = ptile[ln.tab0 + j];
-            tab[pt.f + (size_t)k * pt.stride + lane] = on ? wlambda[ln.toff + lt] * wphi / kHC : 0.0;     // :451
-        }
-    }
+    MALI_COMPUTE_PHI_BODY();
 }
 
 // --------------------------------------------------------------------------------------------------------
@@ -848,14 +856,14 @@ __device__ __forceinline__ double coll_table(const AtomLevels &A, int c, double 
     return out;
 }
 
+// atom a at depth k of column c of the call's inputs (column col0 + c of colconst / pops); shared with
+// mali_perturb_columns (mali_perturb.cuh)
 template <int NLMAX>
-__global__ void setup_levels_kernel(const AtomLevels A, int N, const double *T, const double *ne, const double *vturb,
-                                    double *colconst, int64_t colStride, int64_t off_C, int64_t off_nTotal, double *nStar,
-                                    double *vBroad, double *pops, int64_t popStride, int sumNlevel, int col0)
+__device__ __forceinline__ void setup_levels_point(const AtomLevels &A, int N, const double *T, const double *ne,
+                                                   const double *vturb, double *colconst, int64_t colStride, int64_t off_C,
+                                                   int64_t off_nTotal, double *nStar, double *vBroad, double *pops,
+                                                   int64_t popStride, int sumNlevel, int col0, int a, int c, int k)
 {
-    const int k = blockIdx.x * blockDim.x + threadIdx.x;
-    if (k >= N) return;
-    const int a = blockIdx.y, c = blockIdx.z;
     const double t = T[(size_t)c * N + k], xne = ne[(size_t)c * N + k], vt = vturb[(size_t)c * N + k];
     double *cc = colconst + (size_t)(col0 + c) * colStride;
     const double nTot = cc[off_nTotal + (size_t)a * N + k];
@@ -908,6 +916,16 @@ __global__ void setup_levels_kernel(const AtomLevels A, int N, const double *T, 
     // ---- v_broad, atomic_model.py:241-245
     vBroad[((size_t)c * A.Natom + a) * N + k] = sqrt(A.vTherm[a] * t + vt * vt);
 }
+template <int NLMAX>
+__global__ void setup_levels_kernel(const AtomLevels A, int N, const double *T, const double *ne, const double *vturb,
+                                    double *colconst, int64_t colStride, int64_t off_C, int64_t off_nTotal, double *nStar,
+                                    double *vBroad, double *pops, int64_t popStride, int sumNlevel, int col0)
+{
+    const int k = blockIdx.x * blockDim.x + threadIdx.x;
+    if (k >= N) return;
+    setup_levels_point<NLMAX>(A, N, T, ne, vturb, colconst, colStride, off_C, off_nTotal, nStar, vBroad, pops, popStride,
+                              sumNlevel, col0, blockIdx.y, blockIdx.z, k);
+}
 
 // g_ij of the continua (rh_method.py:453-454): nStar_i / nStar_j * exp(-(hc/k) / lambda / T), written -- times the
 // cross-section alpha, i.e. as Vji of rh_method.py:285 -- into the slot fields of the tile records.  One block row per (continuum, column); threads run over (wavelength, depth).
@@ -918,6 +936,19 @@ struct GijCont {
 struct GijTile {
     int32_t f, stride;    // depth-0 offset of the continuum's field in that tile's records; record stride
 };
+// wavelength lt of continuum ct at depth k of column c of the call's inputs (tab: that column's table); shared with
+// mali_perturb_columns (mali_perturb.cuh)
+__device__ __forceinline__ void setup_gij_point(const GijCont &ct, const GijTile *gt, const double *wavelength,
+                                                const double *alpha, int N, int Lw, const double *T, const double *ns,
+                                                double *tab, double hc_k, int c, int lt, int k)
+{
+    const int la = ct.Nblue + lt;
+    const int ti = la / Lw, ls = la - ti * Lw;
+    const GijTile g = gt[ct.tab0 + ti - ct.tile0];
+    const double v = ns[(size_t)ct.rowI * N + k] / ns[(size_t)ct.rowJ * N + k] *
+                     exp(-hc_k / wavelength[la] / T[(size_t)c * N + k]);
+    tab[g.f + (size_t)k * g.stride + ls] = v * alpha[ct.toff + lt];     // the field holds Vji = g_ij * alpha (:285)
+}
 __global__ void setup_gij_kernel(const GijCont *conts, const GijTile *gt, const double *wavelength, const double *alpha, int N, int Lw,
                                  int sumNlevel, const double *T, const double *nStar, double *colconst, int64_t colStride,
                                  int64_t offTab, int col0)
@@ -929,12 +960,7 @@ __global__ void setup_gij_kernel(const GijCont *conts, const GijTile *gt, const 
     const double *ns = nStar + (size_t)c * sumNlevel * N;
     for (int idx = blockIdx.x * blockDim.x + threadIdx.x; idx < ct.Nlam * N; idx += gridDim.x * blockDim.x) {
         const int lt = idx / N, k = idx - lt * N;
-        const int la = ct.Nblue + lt;
-        const int ti = la / Lw, ls = la - ti * Lw;
-        const GijTile g = gt[ct.tab0 + ti - ct.tile0];
-        const double v = ns[(size_t)ct.rowI * N + k] / ns[(size_t)ct.rowJ * N + k] *
-                         exp(-hc_k / wavelength[la] / T[(size_t)c * N + k]);
-        tab[g.f + (size_t)k * g.stride + ls] = v * alpha[ct.toff + lt];     // the field holds Vji = g_ij * alpha (:285)
+        setup_gij_point(ct, gt, wavelength, alpha, N, Lw, T, ns, tab, hc_k, c, lt, k);
     }
 }
 
@@ -943,14 +969,25 @@ __global__ void setup_gij_kernel(const GijCont *conts, const GijTile *gt, const 
 // that share their upper level, sum_t Uji_t(lambda, k) with Uji = 2hc/lambda^3 * Vji exactly as uv forms it
 // (rh_method.py:284-286; the slots' fields hold Vji = g_ij * alpha), summed in slot order -- the population-independent part of that level's U and of the group's
 // emissivity.  Runs whenever the g_ij fields of a column are (re)written; one thread per (depth, wavelength of the tile).
-__global__ void cont_group_kernel(const TileDesc *tiles, const SlotDesc *slots, const int32_t *groupTiles,
-                                  const double *twohc, int N, int Nspect, int Lw, double *colconst, int64_t colStride,
-                                  int64_t offTab, int col0)
+// The whole body, shared with mali_perturb_columns (mali_perturb.cuh), which runs one depth of a column: the index
+// policy gives the group tile, the column of the call and the threads' loop over idx = k * Lw + ls, and is read where
+// the kernel read blockIdx / threadIdx when it was a single body, which keeps cont_group_kernel's instructions as they were.
+struct GroupGridIdx {
+    __device__ __forceinline__ unsigned tile() const { return blockIdx.y; }
+    __device__ __forceinline__ unsigned col() const { return blockIdx.z; }
+    __device__ __forceinline__ int first() const { return blockIdx.x * blockDim.x + threadIdx.x; }
+    __device__ __forceinline__ int end(int N, int Lw) const { return N * Lw; }
+    __device__ __forceinline__ int step() const { return gridDim.x * blockDim.x; }
+};
+template <class Ix>
+__device__ __forceinline__ void cont_group_body(const TileDesc *tiles, const SlotDesc *slots, const int32_t *groupTiles,
+                                                const double *twohc, int N, int Nspect, int Lw, double *colconst,
+                                                int64_t colStride, int64_t offTab, int col0, Ix ix)
 {
-    const TileDesc td = tiles[groupTiles[blockIdx.y]];
-    double *tab = colconst + (size_t)(col0 + blockIdx.z) * colStride + offTab + td.recOff;
+    const TileDesc td = tiles[groupTiles[ix.tile()]];
+    double *tab = colconst + (size_t)(col0 + ix.col()) * colStride + offTab + td.recOff;
     const SlotDesc *sl = slots + td.slot0;
-    for (int idx = blockIdx.x * blockDim.x + threadIdx.x; idx < N * Lw; idx += gridDim.x * blockDim.x) {
+    for (int idx = ix.first(); idx < ix.end(N, Lw); idx += ix.step()) {
         const int k = idx / Lw, ls = idx - k * Lw;
         const int la = td.la0 + ls;
         double *rec = tab + (size_t)k * td.stride;
@@ -974,6 +1011,12 @@ __global__ void cont_group_kernel(const TileDesc *tiles, const SlotDesc *slots, 
         }
     }
 }
+__global__ void cont_group_kernel(const TileDesc *tiles, const SlotDesc *slots, const int32_t *groupTiles,
+                                  const double *twohc, int N, int Nspect, int Lw, double *colconst, int64_t colStride,
+                                  int64_t offTab, int col0)
+{
+    cont_group_body(tiles, slots, groupTiles, twohc, N, Nspect, Lw, colconst, colStride, offTab, col0, GroupGridIdx{});
+}
 
 // --------------------------------------------------------------------------------------------------------
 // Background / EOS on the device (SURVEY.md 8f rank 1): Background.compute_background_eos (background.py:21-53) and the
@@ -990,10 +1033,9 @@ constexpr int kEosWork = 20;   // pgas, pe, chi_c (per m at 5000 A), then the 17
 
 // one thread per (column, depth): gas and electron pressure from (T, rho), the background partial densities, and the
 // 5000 A opacity the scale conversion needs
-__global__ void eos_kernel(const EosParams P, int N, int ncol, const double *T, const double *nHTot, double *work)
+// point idx = c * N + k of the call's inputs; shared with mali_perturb_columns (mali_perturb.cuh)
+__device__ __forceinline__ void eos_point(const EosParams &P, const double *T, const double *nHTot, double *work, int idx)
 {
-    const int idx = blockIdx.x * blockDim.x + threadIdx.x;
-    if (idx >= N * ncol) return;
     const double t = T[idx];
     const double rho = P.amu_wph * nHTot[idx] * P.cm3 / P.g_to_kg;                       // background.py:33
     double *w = work + (size_t)idx * kEosWork;
@@ -1009,17 +1051,21 @@ __global__ void eos_kernel(const EosParams P, int N, int ncol, const double *T, 
     eos::cop_one(t, TKEV, HTK, TLOG, xne, 5000.0, w + 3, op, sc);
     w[2] = op / P.cm_to_m;                                                                // atmosphere.py:92
 }
+__global__ void eos_kernel(const EosParams P, int N, int ncol, const double *T, const double *nHTot, double *work)
+{
+    const int idx = blockIdx.x * blockDim.x + threadIdx.x;
+    if (idx >= N * ncol) return;
+    eos_point(P, T, nHTot, work, idx);
+}
 
 // one thread per (column, wavelength, depth): chi = cop / CM_TO_M, eta = planck(T, lambda) * chi (utils.py:17-22 as numpy
-// evaluates it for an array of wavelengths), sca = ne * sigma_T  -- written into the bg fields of the tile records
-__global__ void background_kernel(const EosParams P, const TileDesc *tiles, const double *wavelength, int N, int Nspect,
-                                  int Lw, const double *T, const double *ne, const double *work, double *colconst,
-                                  int64_t colStride, int64_t offTab, int col0)
+// evaluates it for an array of wavelengths), sca = ne * sigma_T  -- written into the bg fields of the tile records.
+// One thread's work; shared with mali_perturb_columns (mali_perturb.cuh).
+__device__ __forceinline__ void background_point(const EosParams &P, const TileDesc *tiles, const double *wavelength, int N,
+                                                 int Nspect, int Lw, const double *T, const double *ne, const double *work,
+                                                 double *colconst, int64_t colStride, int64_t offTab, int col0, int c,
+                                                 int la, int k)
 {
-    const int c = blockIdx.z;
-    const int la = blockIdx.y;
-    const int k = blockIdx.x * blockDim.x + threadIdx.x;
-    if (k >= N) return;
     const size_t idx = (size_t)c * N + k;
     const double t = T[idx];
     const double *w = work + idx * kEosWork;
@@ -1045,6 +1091,16 @@ __global__ void background_kernel(const EosParams P, const TileDesc *tiles, cons
             f[Lw + q - ls] = eta;
             f[2 * Lw + q - ls] = ne[idx] * P.thomson;
         }
+}
+__global__ void background_kernel(const EosParams P, const TileDesc *tiles, const double *wavelength, int N, int Nspect,
+                                  int Lw, const double *T, const double *ne, const double *work, double *colconst,
+                                  int64_t colStride, int64_t offTab, int col0)
+{
+    const int c = blockIdx.z;
+    const int la = blockIdx.y;
+    const int k = blockIdx.x * blockDim.x + threadIdx.x;
+    if (k >= N) return;
+    background_point(P, tiles, wavelength, N, Nspect, Lw, T, ne, work, colconst, colStride, offTab, col0, c, la, k);
 }
 
 // one thread per column: the column-mass branch of convert_scales (atmosphere.py:94-111): heights from the column

@@ -9,6 +9,7 @@ radiative model, and drives libmali_b200.so through its C ABI.
     I = eng.compute_rays([1.0, 0.5])                      # [ncol, Nspect, nmu] emergent intensity at user angles
     d = eng.compute_rays_depth([1.0, 0.5])                # RayDepthData: I, chi, S, tau, contrib per depth, z_tau1
     r = eng.compute_rates()                               # RadiativeRates: Rij, Rji, net [ncol, Ntrans, Nspace]
+    rf = eng.compute_response(base, 'temperature', 25.0, aDamp_minus=.., aDamp_plus=..)   # ResponseFunction
 
 Columns are independent (no cross-column arithmetic anywhere), which is what makes the path data-parallel:
 ranks of a multi-GPU job each own a contiguous slice of columns (see lightspinner_b200/sharding.py).
@@ -582,15 +583,147 @@ class MaliEngine:
         self._raise_rays_faults(col0)
         return res
 
-    def reset_iteration_state(self):
-        self.t_iter.zero_()
-        self.t_done.zero_()
-        self.t_dPops.fill_(1.0)
-        self.t_dJ.fill_(1.0)
-        self.t_status.zero_()
+    # ------------------------------------------------------------------ response functions
+    def compute_response(self, base, param, step, *, aDamp_minus=None, aDamp_plus=None, depths=None, mus=None,
+                         max_iter=500, tolJ=2e-3, tolPops=1e-3, col0=0, ncol=None):
+        """Response function of the emergent intensity to `param` ('temperature' K, 'vturb' or 'vlos' m/s) at every
+        depth in `depths` (default all), by central differences with step `step` (response_fn.py; definition in
+        include/mali_b200.h at mali_perturb_columns and DESIGN.md): a ResponseFunction.
+
+        base: an upload_thermo problem dict (temperature, ne, nHTot, vturb, vlos, nTotal, aDamp and cmass or height),
+        solved from LTE, or from base['n'] if given.  aDamp_minus / aDamp_plus [Ntrans, Nspace]: the damping of the
+        base atmosphere with `param` shifted by -step / +step at every depth (required for 'temperature' and 'vturb',
+        not used for 'vlos').  Every perturbed column starts from the solved base's populations with J = 0 and runs
+        the loop of iterate_async (per-column convergence at tolJ / tolPops, at most max_iter iterations, the engine's
+        Ng option).  mus: the angles of compute_rays for I, or None for I at the quadrature angles after each loop.
+
+        Columns [col0, col0+ncol) (default: all from col0) are the workspace and everything in them is overwritten:
+        col0 holds the base as set up, col0 + 1 the base solve, the rest take the perturbed columns in chunks, each
+        formed from col0 by mali_perturb_columns.  At least 3 columns.  Needs set_eos() and set_atoms().  Raises
+        LinAlgError / FloatingPointError as raise_on_faults does."""
+        from .response import ResponseFunction, base_arrays, response_args
+        if getattr(self, '_eos_tables', None) is None or getattr(self, '_atom_tables', None) is None:
+            raise ValueError('compute_response needs set_eos() and set_atoms()')
+        mt = self.mt
+        N, S = mt.Nspace, mt.Nspect
+        col0 = int(col0)
+        ncol = self.ncol - col0 if ncol is None else int(ncol)
+        if col0 < 0 or ncol < 1 or col0 + ncol > self.ncol:
+            raise ValueError('columns [%d, %d) outside the batch of %d' % (col0, col0 + ncol, self.ncol))
+        if ncol < 3:
+            raise ValueError('the workspace needs at least 3 columns (the base as set up, the base solve and one '
+                             'perturbed column), got %d' % ncol)
+        step, depths, adm, adp = response_args(param, step, aDamp_minus, aDamp_plus, depths, N, mt.Ntrans)
+        b = base_arrays(base, N, mt.Natom, mt.Ntrans)
+        if mus is not None:
+            mus = rays_angles(mus)
+        if int(max_iter) < 1:
+            raise ValueError('max_iter must be >= 1, got %r' % (max_iter,))
+        src, bcol, w0, W = col0, col0 + 1, col0 + 2, ncol - 2
+
+        # the source column: set up once, never iterated; the base solve beside it
+        self.upload_thermo([b], src)
+        src_work = self._last_work
+        if 'n' in base:
+            b['n'] = base['n']
+        self.upload_thermo([b], bcol, start_from_lte='n' not in base)
+        self._solve_range(bcol, 1, max_iter, tolJ, tolPops)
+        I0 = self._response_intensity(mus, bcol, 1)[0]
+        base_iter, base_conv = int(self.t_iter[bcol].item()), bool(self.t_done[bcol].item() == 1)
+
+        pops0 = self.t_pops[bcol * self.lay.pops:(bcol + 1) * self.lay.pops]
+        cols = [(int(d), s) for d in depths for s in (-1, 1)]
+        nd = depths.shape[0]
+        nmu = mt.Nrays if mus is None else mus.shape[0]
+        I = np.empty((nd, 2, S, nmu))
+        its = np.empty((nd, 2), dtype=np.int64)
+        conv = np.empty((nd, 2), dtype=bool)
+        for i0 in range(0, len(cols), W):
+            chunk = cols[i0:i0 + W]
+            nc = len(chunk)
+            self._perturb_chunk(b, param, step, chunk, adm, adp, src, src_work, pops0, w0)
+            self._solve_range(w0, nc, max_iter, tolJ, tolPops)
+            Ic = self._response_intensity(mus, w0, nc)
+            it = self.t_iter[w0:w0 + nc].cpu().numpy()
+            dn = self.t_done[w0:w0 + nc].cpu().numpy()
+            for q, (k, s) in enumerate(chunk):
+                d, j = (i0 + q) // 2, (s + 1) // 2
+                I[d, j], its[d, j], conv[d, j] = Ic[q], it[q], dn[q] == 1
+        return ResponseFunction(param=param, step=step, depths=depths, mu=mus, rf=(I[:, 1] - I[:, 0]) / (2.0 * step),
+                                I_minus=I[:, 0], I_plus=I[:, 1], I0=I0, iterations=its, converged=conv,
+                                base_iterations=base_iter, base_converged=base_conv)
+
+    def _perturb_chunk(self, b, param, step, chunk, adm, adp, src, src_work, pops0, w0):
+        """Columns [w0, w0+len(chunk)) become the columns (k, s) of `chunk` (mali_perturb_columns from the source column
+        `src`, set up from the base arrays `b` by upload_thermo, whose EOS work rows are `src_work`), starting from the
+        populations pops0; their profile inputs are kept for compute_rays."""
+        from .response import perturbed_bbc, perturbed_value
+        from .tables import planck_bc
+        mt, N, SL = self.mt, self.mt.Nspace, int(self.lay.sumNlevel)
+        nc = len(chunk)
+        dev = lambda a: torch.as_tensor(np.ascontiguousarray(a), dtype=torch.float64).to(self.device)
+        P = lambda t: C.c_void_p(t.data_ptr()) if t is not None else None
+        keys = ('temperature', 'ne', 'nHTot', 'vturb', 'vlos') + (('cmass',) if 'cmass' in b else ())
+        # the base repeated, plus one indexed write per column
+        ins = {k: dev(b[k]).reshape(1, N).repeat(nc, 1) for k in keys}
+        ks = np.array([k for k, _ in chunk], dtype=np.int32)
+        ar = torch.arange(nc, device=self.device)
+        kt = torch.as_tensor(ks, dtype=torch.int64, device=self.device)
+        x = b[param]
+        ins[param][ar, kt] = dev([perturbed_value(x, step, k, s) for k, s in chunk])
+        aD = dev(b['aDamp']).reshape(1, mt.Ntrans, N).repeat(nc, 1, 1)
+        if param != 'vlos':
+            aD[ar, :, kt] = dev(np.stack([(adp if s > 0 else adm)[:, k] for k, s in chunk]))
+        bbc = None
+        if param == 'temperature':
+            bbc0 = planck_bc(mt.wavelength, x)
+            bbc = dev(np.stack([bb if bb is not None else bbc0 for bb in
+                                (perturbed_bbc(mt.wavelength, x, param, step, k, s) for k, s in chunk)]))
+        aD, vBroad, vlos = self._keep_profile_inputs(w0, nc, aD, self.t_vBroad[w0:w0 + nc], ins['vlos'])
+        work = torch.empty(nc * N * 21, dtype=torch.float64, device=self.device)
+        desc = _capi.PerturbDesc(ks.ctypes.data_as(C.POINTER(C.c_int32)),
+                                 *(P(ins[k]) for k in ('temperature', 'ne', 'nHTot', 'vturb')), P(vlos),
+                                 P(ins.get('cmass')), P(aD), P(bbc), P(pops0), P(src_work),
+                                 P(self.nStar[src * SL * N:(src + 1) * SL * N]), P(self.t_vBroad[src]), P(work),
+                                 P(self.nStar[w0 * SL * N:(w0 + nc) * SL * N]), P(vBroad))
+        with torch.cuda.device(self.device):
+            self._check(self.lib.mali_perturb_columns(self._handle, C.byref(self.bufs), src, w0, nc, C.byref(desc),
+                                                      self._stream()))
+        torch.cuda.current_stream(self.device).synchronize()    # (the inputs above are freed on return)
+
+    def _solve_range(self, col0, ncol, max_iter, tolJ, tolPops):
+        """Fresh iteration state for columns [col0, col0+ncol), then the device loop in rounds of 16 iterations until
+        every column is done or max_iter iterations ran; raises as raise_on_faults."""
+        self.reset_iteration_state(col0, ncol)
+        left = int(max_iter)
+        while left > 0:
+            n = min(16, left)
+            self.iterate_async(n, tolJ, tolPops, col0, ncol)
+            left -= n
+            if bool((self.t_done[col0:col0 + ncol] != 0).all().item()):
+                break
+        self.raise_on_faults(col0, ncol)
+
+    def _response_intensity(self, mus, col0, ncol):
+        """[ncol, Nspect, nmu]: I of the last formal solution (mus None) or compute_rays at mus."""
+        if mus is None:
+            L = self.lay.I
+            return self.t_I[col0 * L:(col0 + ncol) * L].view(ncol, self.mt.Nspect, self.mt.Nrays).cpu().numpy()
+        return self.compute_rays(mus, col0, ncol)
+
+    def reset_iteration_state(self, col0=0, ncol=None):
+        """Fresh loop state (iterations, done, dPops, dJ, status and the Ng history) for columns [col0, col0+ncol),
+        default all."""
+        ncol = self.ncol - col0 if ncol is None else ncol
+        c = slice(col0, col0 + ncol)
+        self.t_iter[c].zero_()
+        self.t_done[c].zero_()
+        self.t_dPops[c].fill_(1.0)
+        self.t_dJ[c].fill_(1.0)
+        self.t_status[c].zero_()
         if self.ng is not None:
-            self.t_ng_nse.zero_()
-            self.t_ng_accepted.zero_()
+            self.t_ng_nse[c].zero_()
+            self.t_ng_accepted[col0 * self.mt.Natom:(col0 + ncol) * self.mt.Natom].zero_()
 
     def ng_reset(self, col0=0, ncol=None):
         """Restart the Ng history of columns [col0, col0+ncol): needed after their populations were edited between
